@@ -6,10 +6,12 @@
 // contact joins them.  A connected component of its graph — an "island": static bodies united through this substep's
 // contacts — is an independent linear system, and nearly all of them are small (a free body; a column of stacked
 // boxes).  So instead of a grid-wide CG whose every iteration streams the whole matrix from HBM and synchronises the
-// device twice, every island is solved by its own team (a warp or one CTA) that keeps the island's matrix, the
-// inverses of its preconditioner blocks and the CG vectors in shared memory for the whole solve, iterates with team
-// barriers only, and stops on its own residual:  ||r_island|| <= tol ||b_island||  per coordinate column (a stricter
-// test than the same bound on the global norms).  Only islands too large for one CTA go to the grid-wide CG (pcg.cu).
+// device twice, every island is solved by its own team and stops on its own residual:  ||r_island|| <= tol ||b_island||
+// per coordinate column (a stricter test than the same bound on the global norms).  An island that is one
+// preconditioner block is refined by one warp with its exact block inverse, a small one by one CTA with its dense
+// inverse; the CG team is one CTA that keeps the island's matrix, the inverses of its preconditioner blocks and the CG
+// vectors in shared memory for the whole solve and iterates with CTA barriers only.  Only islands too large for one CTA
+// go to the grid-wide CG (pcg.cu).
 //
 // Determinism: the island order (bodies ascending inside an island, nodes ascending inside a body) comes from a
 // stable sort, every dot product is reduced in a fixed order inside the team, no float atomics.
@@ -179,21 +181,21 @@ __global__ void __launch_bounds__(kThreads) k_isl_compact(uint32_t n, const uint
 // ------------------------------------------------------------------------------------------------ solver ----
 struct IslandLayout { uint32_t r, p, val, inv, blkOff, blkSrc, col, members, leader, blkM, red, ctr, total; };
 
-static IslandLayout islandLayout(const IslandCaps& c, int team, bool matSmem) {
+static IslandLayout islandLayout(const IslandCaps& c) {
   IslandLayout L{};
   uint32_t off = 0;
   auto take = [&](uint32_t bytes) { uint32_t at = off; off += (bytes + 15u) & ~15u; return at; };
   L.r = take(16u * c.maxNodes);
   L.p = take(16u * c.maxNodes);
-  L.val = take(matSmem ? 4u * c.maxNnz : 0u);
+  L.val = take(4u * c.maxNnz);
   L.inv = take(4u * c.maxInv);
   L.blkOff = take(4u * c.maxBlocks);
   L.blkSrc = take(4u * c.maxBlocks);
-  L.col = take(matSmem ? 2u * c.maxNnz : 0u);
+  L.col = take(2u * c.maxNnz);
   L.members = take(64u * c.maxBlocks);
   L.leader = take(c.maxBlocks ? 2u * c.maxNodes : 0u);
   L.blkM = take(c.maxBlocks);
-  L.red = take(team > 32 ? 2u * 9u * 32u * 4u : 0u);
+  L.red = take(2u * 9u * 32u * 4u);
   L.ctr = take(16u);
   L.total = off;
   return L;
@@ -214,18 +216,12 @@ struct IslandArgs {
   uint4* trace;                // diagnostics: per list entry (rows, iterations, clocks, matrix entries), or null
 };
 
-template <int TEAM>
-__device__ __forceinline__ void teamSync() {
-  if (TEAM == 32) __syncwarp(); else __syncthreads();
-}
-
-// Fixed-order sum of K values per thread over the team; every thread gets the result.  CTA teams alternate between
-// two scratch buffers, so one barrier per reduction is enough.
+// Fixed-order sum of K values per thread over the CTA; every thread gets the result.  The CTA alternates between two
+// scratch buffers, so one barrier per reduction is enough.
 template <int TEAM, int K>
 __device__ __forceinline__ void teamReduce(float (&v)[K], float* __restrict__ sRed, int& phase, int tid) {
 #pragma unroll
   for (int k = 0; k < K; ++k) v[k] = warpSum(v[k]);
-  if (TEAM == 32) return;
   float* buf = sRed + phase * (9 * 32);
   phase ^= 1;
   const int lane = tid & 31, warp = tid >> 5;
@@ -241,54 +237,55 @@ __device__ __forceinline__ void teamReduce(float (&v)[K], float* __restrict__ sR
   }
 }
 
-// SPLIT > 1: every row is shared by SPLIT neighbouring lanes (matrix entries and preconditioner terms strided over them,
-// partial sums combined by shuffles) — for a short list of mid-size islands, where the solve waits for the dependent
-// shared-memory loads of its one slowest island and more, shorter instruction streams are what helps.
-template <int SPLIT>
-__device__ __forceinline__ void splitSum3(float (&v)[3]) {
-#pragma unroll
-  for (int o = SPLIT / 2; o > 0; o >>= 1) {
-#pragma unroll
-    for (int c = 0; c < 3; ++c) v[c] += __shfl_xor_sync(0xffffffffu, v[c], o);
+// The three-column convergence test of every island solve: ||r|| <= tol ||b|| per coordinate column, squared.
+__device__ __forceinline__ bool converged3(const float (&rr)[3], const float (&bb)[3], float tol2) {
+  return rr[0] <= tol2 * bb[0] + 1e-36f && rr[1] <= tol2 * bb[1] + 1e-36f && rr[2] <= tol2 * bb[2] + 1e-36f;
+}
+
+// One island's entry in its solve's 4-word statistics record (IslandWork::solveStats, read by the host once per tick):
+// max iterations, iterations x 32-row units, islands stopped at the cap and their worst relative residual.
+__device__ __forceinline__ void recordSolve(uint32_t* stats, uint32_t iters, uint32_t m, bool conv, const float (&rr)[3],
+                                            const float (&bb)[3]) {
+  atomicMax(stats, iters);
+  atomicAdd(stats + 1, iters * ((m + 31u) >> 5));
+  if (!conv) {
+    float rel = 0.0f;
+    for (int c = 0; c < 3; ++c) if (bb[c] > 0.0f) rel = fmaxf(rel, rr[c] / bb[c]);
+    atomicAdd(stats + 2, 1u);
+    atomicMax(stats + 3, __float_as_uint(sqrtf(rel)));
   }
 }
 
-template <int TEAM, int RPT, bool MAT_SMEM, int SPLIT = 1>
-__global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEAM <= 128 ? 5 : (TEAM <= 320 ? 2 : 1))) k_island_pcg(IslandArgs a, IslandLayout L, IslandCaps caps, int tier) {
-  static_assert(SPLIT == 1 || (TEAM > 32 && (32 % SPLIT) == 0), "lanes of a row sit in one warp");
-  constexpr int ROWS = TEAM / SPLIT;   // rows per pass of the team
+// One CTA of TEAM threads per island, RPT rows per thread.
+template <int TEAM, int RPT>
+__global__ void __launch_bounds__(TEAM, TEAM <= 128 ? 5 : (TEAM <= 320 ? 2 : 1)) k_island_pcg(IslandArgs a, IslandLayout L, IslandCaps caps, int tier) {
   extern __shared__ __align__(16) unsigned char islSmem[];
-  constexpr int kTeams = TEAM == 32 ? 8 : 1;
-  using ColT = typename std::conditional<MAT_SMEM, uint16_t, int>::type;
-  const int team = TEAM == 32 ? (int)(threadIdx.x >> 5) : 0;
-  const int tid = TEAM == 32 ? (int)(threadIdx.x & 31) : (int)threadIdx.x;
-  const int sub = tid % SPLIT, rt = tid / SPLIT;   // lane of the row, row of the pass
-  unsigned char* base = islSmem + (size_t)team * L.total;
-  float4* sR = reinterpret_cast<float4*>(base + L.r);
-  float4* sP = reinterpret_cast<float4*>(base + L.p);
-  float* sInv = reinterpret_cast<float*>(base + L.inv);
-  uint32_t* sBlkOff = reinterpret_cast<uint32_t*>(base + L.blkOff);
-  uint32_t* sBlkSrc = reinterpret_cast<uint32_t*>(base + L.blkSrc);
-  uint16_t* sMem = reinterpret_cast<uint16_t*>(base + L.members);
-  uint16_t* sLeader = reinterpret_cast<uint16_t*>(base + L.leader);
-  uint8_t* sBlkM = reinterpret_cast<uint8_t*>(base + L.blkM);
-  float* sRed = reinterpret_cast<float*>(base + L.red);
-  uint32_t* sCtr = reinterpret_cast<uint32_t*>(base + L.ctr);
+  const int tid = (int)threadIdx.x;
+  float4* sR = reinterpret_cast<float4*>(islSmem + L.r);
+  float4* sP = reinterpret_cast<float4*>(islSmem + L.p);
+  float* sInv = reinterpret_cast<float*>(islSmem + L.inv);
+  uint32_t* sBlkOff = reinterpret_cast<uint32_t*>(islSmem + L.blkOff);
+  uint32_t* sBlkSrc = reinterpret_cast<uint32_t*>(islSmem + L.blkSrc);
+  uint16_t* sMem = reinterpret_cast<uint16_t*>(islSmem + L.members);
+  uint16_t* sLeader = reinterpret_cast<uint16_t*>(islSmem + L.leader);
+  uint8_t* sBlkM = reinterpret_cast<uint8_t*>(islSmem + L.blkM);
+  float* sRed = reinterpret_cast<float*>(islSmem + L.red);
+  uint32_t* sCtr = reinterpret_cast<uint32_t*>(islSmem + L.ctr);
   const uint32_t count = a.counts[1 + tier];
   const uint4* descs = a.tierDesc + (size_t)tier * a.listStride;
   int phase = 0;
-  const uint32_t stride = gridDim.x * kTeams;
-  uint32_t wi = blockIdx.x * kTeams + team;
+  const uint32_t stride = gridDim.x;
+  uint32_t wi = blockIdx.x;
   uint4 descNext = wi < count ? __ldg(descs + wi) : make_uint4(0u, 0u, 0u, 0u);
   for (; wi < count; wi += stride) {
     const uint4 desc = descNext;
     if (wi + stride < count) descNext = __ldg(descs + wi + stride);  // in flight while this island is solved
     const uint32_t s0 = desc.y, m = desc.z, z0 = desc.w;
     const long long t0 = a.trace ? clock64() : 0ll;
-    float* mv = MAT_SMEM ? reinterpret_cast<float*>(base + L.val) : a.matVal + z0;
-    ColT* mc = MAT_SMEM ? reinterpret_cast<ColT*>(base + L.col) : reinterpret_cast<ColT*>(a.matCol + z0);
+    float* mv = reinterpret_cast<float*>(islSmem + L.val);
+    uint16_t* mc = reinterpret_cast<uint16_t*>(islSmem + L.col);
     if (tid == 0) { sCtr[0] = 0; sCtr[1] = 0; }
-    teamSync<TEAM>();
+    __syncthreads();
     // ---- stage the island.  Rows are re-indexed without a gather per entry: S never leaves a body and the island order
     //      keeps a body's nodes together by rank, so local column = (row's body base) + rank of the column (host table).
     //      x of the island goes to sP and b to sR for the start residual below.
@@ -297,7 +294,7 @@ __global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEA
     float red9[9] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};  // r.z (3), r.r (3), b.b (3)
 #pragma unroll
     for (int k = 0; k < RPT; ++k) {
-      const uint32_t l = (uint32_t)rt + (uint32_t)k * ROWS;
+      const uint32_t l = (uint32_t)tid + (uint32_t)k * TEAM;
       rs[k] = 0; rn[k] = 0; rb[k] = 0xffffffffu; slot[k] = 0; gid[k] = 0; cdg[k] = 0.0f;
       dl[k][0] = dl[k][1] = dl[k][2] = 0.0f;
       if (l >= m) continue;
@@ -308,48 +305,29 @@ __global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEA
       const int kk0 = a.rowPtr[g], kk1 = a.rowPtr[g + 1];
       const uint32_t bodyBase = l - a.rankInBody[g];
       const float4 bi = a.b[g];
-      if (sub == 0) { sP[l] = a.x[g]; sR[l] = bi; }
+      sP[l] = a.x[g]; sR[l] = bi;
       cdg[k] = a.cDiag ? a.cDiag[g] : 0.0f;
       const uint32_t sl = a.slotOf[g];
       slot[k] = sl;
+      // (putting the loads of eight entries in flight together helped the staged warp tier, r02g: 85 -> 75 us; on a
+      // CTA it costs registers and 10 %)
       uint32_t e = rstart;
-      if (TEAM == 32) {
-        // warp tier: the island is staged by one warp whose only other work is waiting, so all 16 loads of eight entries
-        // are put in flight together (r02g: 85 -> 75 us); on the CTA tiers the same batching cost registers and 10 %
-        for (int kk = kk0; kk < kk1; kk += 8) {
-          uint32_t rk[8];
-          float vv[8];
-#pragma unroll
-          for (int j = 0; j < 8; ++j)
-            if (kk + j < kk1) { rk[j] = __ldg(a.colRank + kk + j); vv[j] = __ldg(a.val + kk + j); }
-#pragma unroll
-          for (int j = 0; j < 8; ++j)
-            if (kk + j < kk1) {
-              const bool out = rk[j] == 0xffffffffu;  // an explicit zero pointing outside the body (bend stencils): dropped
-              mc[e] = (ColT)(out ? l : bodyBase + rk[j]);
-              mv[e] = out ? 0.0f : vv[j];
-              ++e;
-            }
-        }
-      } else {
 #pragma unroll 4
-        for (int kk = kk0 + sub; kk < kk1; kk += SPLIT) {
-          const uint32_t rk = __ldg(a.colRank + kk);
-          const float v = __ldg(a.val + kk);
-          const bool out = rk == 0xffffffffu;
-          mc[e + (kk - kk0)] = (ColT)(out ? l : bodyBase + rk);
-          mv[e + (kk - kk0)] = out ? 0.0f : v;
-        }
-        e += (uint32_t)(kk1 - kk0);
+      for (int kk = kk0; kk < kk1; ++kk) {
+        const uint32_t rk = __ldg(a.colRank + kk);
+        const float v = __ldg(a.val + kk);
+        const bool out = rk == 0xffffffffu;  // an explicit zero pointing outside the body (bend stencils): dropped
+        mc[e + (kk - kk0)] = (uint16_t)(out ? l : bodyBase + rk);
+        mv[e + (kk - kk0)] = out ? 0.0f : v;
       }
+      e += (uint32_t)(kk1 - kk0);
       if (a.cPtr) {
         const int c0 = a.cPtr[g], c1 = a.cPtr[g + 1];
-        for (int kk = c0 + sub; kk < c1; kk += SPLIT) {
-          mc[e + (kk - c0)] = (ColT)(__ldg(a.pos + __ldg(a.cCol + kk)) - s0);
+        for (int kk = c0; kk < c1; ++kk) {
+          mc[e + (kk - c0)] = (uint16_t)(__ldg(a.pos + __ldg(a.cCol + kk)) - s0);
           mv[e + (kk - c0)] = __ldg(a.cVal + kk);
         }
       }
-      if (sub != 0) continue;   // the row's bookkeeping below belongs to its first lane
       red9[6] += bi.x * bi.x; red9[7] += bi.y * bi.y; red9[8] += bi.z * bi.z;
       a.blkLocal[sl] = l;
       if (caps.maxBlocks) {
@@ -366,48 +344,36 @@ __global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEA
         }
       }
     }
-    teamSync<TEAM>();
+    __syncthreads();
     // start residual r = b - A x from shared memory, accumulated in fp64 (float products are exact in double): b and A x
     // agree to ~7 digits and the difference is what matters
 #pragma unroll
     for (int k = 0; k < RPT; ++k) {
-      const uint32_t l = (uint32_t)rt + (uint32_t)k * ROWS;
-      const bool act = l < m;
-      if (SPLIT == 1 && !act) continue;
-      double y0 = 0.0, y1 = 0.0, y2 = 0.0;
-      if (act) {
-        if (sub == 0) {
-          const float4 xi = sP[l];
-          y0 = (double)cdg[k] * (double)xi.x; y1 = (double)cdg[k] * (double)xi.y; y2 = (double)cdg[k] * (double)xi.z;
-        }
-        const uint32_t e1 = rs[k] + rn[k];
+      const uint32_t l = (uint32_t)tid + (uint32_t)k * TEAM;
+      if (l >= m) continue;
+      const float4 xi = sP[l];
+      double y0 = (double)cdg[k] * (double)xi.x, y1 = (double)cdg[k] * (double)xi.y, y2 = (double)cdg[k] * (double)xi.z;
+      const uint32_t e1 = rs[k] + rn[k];
 #pragma unroll 4
-        for (uint32_t e = rs[k] + sub; e < e1; e += SPLIT) {
-          const double v = (double)mv[e];
-          const float4 xv = sP[mc[e]];
-          y0 += v * (double)xv.x; y1 += v * (double)xv.y; y2 += v * (double)xv.z;
-        }
+      for (uint32_t e = rs[k]; e < e1; ++e) {
+        const double v = (double)mv[e];
+        const float4 xv = sP[mc[e]];
+        y0 += v * (double)xv.x; y1 += v * (double)xv.y; y2 += v * (double)xv.z;
       }
-#pragma unroll
-      for (int o = SPLIT / 2; o > 0; o >>= 1) {
-        y0 += __shfl_xor_sync(0xffffffffu, y0, o); y1 += __shfl_xor_sync(0xffffffffu, y1, o); y2 += __shfl_xor_sync(0xffffffffu, y2, o);
-      }
-      if (act && sub == 0) {
-        const float4 bi = sR[l];
-        sR[l] = make_float4((float)((double)bi.x - y0), (float)((double)bi.y - y1), (float)((double)bi.z - y2), 0.0f);
-      }
+      const float4 bi = sR[l];
+      sR[l] = make_float4((float)((double)bi.x - y0), (float)((double)bi.y - y1), (float)((double)bi.z - y2), 0.0f);
     }
-    teamSync<TEAM>();
+    __syncthreads();
     if (caps.maxBlocks) {
 #pragma unroll
       for (int k = 0; k < RPT; ++k) {
-        const uint32_t l = (uint32_t)rt + (uint32_t)k * ROWS;
+        const uint32_t l = (uint32_t)tid + (uint32_t)k * TEAM;
         if (l >= m) continue;
         const uint32_t lead = a.pos[a.blockNodes[(slot[k] >> 5) * 32]] - s0;
         const uint32_t idx = sLeader[lead];
         if (idx != 0xffffu) { rb[k] = (idx << 5) | (slot[k] & 31u); sMem[idx * 32 + (slot[k] & 31u)] = (uint16_t)l; }
       }
-      teamSync<TEAM>();
+      __syncthreads();
       // inverses: one warp per block, 16 B per lane and step
       const uint32_t nBlk = min(sCtr[0], caps.maxBlocks);
       for (uint32_t idx = (uint32_t)tid >> 5; idx < nBlk; idx += TEAM / 32) {
@@ -419,7 +385,7 @@ __global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEA
         for (uint32_t t = (uint32_t)tid & 31u; t < size4; t += 32u) dst[t] = __ldg(src + t);
       }
     }
-    teamSync<TEAM>();
+    __syncthreads();
 
     // z = Minv r for one of this thread's rows
     auto precond = [&](int k, float (&z)[3]) {
@@ -429,32 +395,22 @@ __global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEA
         const int lane = (int)(rb[k] & 31u), mB = (int)sBlkM[idx];
         const float* inv = sInv + sBlkOff[idx];
         const uint16_t* mem = sMem + idx * 32;
-        if (SPLIT == 1) {
-          int off = lane * (lane + 1) / 2;
+        int off = lane * (lane + 1) / 2;
 #pragma unroll 3
-          for (int j = 0; j < mB; ++j) {
-            const float w = inv[off];
-            const float4 rj = sR[mem[j]];
-            z[0] = fmaf(w, rj.x, z[0]); z[1] = fmaf(w, rj.y, z[1]); z[2] = fmaf(w, rj.z, z[2]);
-            off += j < lane ? 1 : j + 1;
-          }
-        } else {   // this lane's share of the row: terms sub, sub + SPLIT, ...
-          const int tri = lane * (lane + 1) / 2;
-#pragma unroll 2
-          for (int j = sub; j < mB; j += SPLIT) {
-            const float w = inv[j < lane ? tri + j : j * (j + 1) / 2 + lane];
-            const float4 rj = sR[mem[j]];
-            z[0] = fmaf(w, rj.x, z[0]); z[1] = fmaf(w, rj.y, z[1]); z[2] = fmaf(w, rj.z, z[2]);
-          }
+        for (int j = 0; j < mB; ++j) {
+          const float w = inv[off];
+          const float4 rj = sR[mem[j]];
+          z[0] = fmaf(w, rj.x, z[0]); z[1] = fmaf(w, rj.y, z[1]); z[2] = fmaf(w, rj.z, z[2]);
+          off += j < lane ? 1 : j + 1;
         }
-      } else {  // block not resident (tier 3, or the island has more blocks than the tier's table): same sum from global memory
+      } else {  // block not resident (the island has more blocks than the tier's table): same sum from global memory
         const uint32_t b = slot[k] >> 5;
         const int lane = (int)(slot[k] & 31u);
         const uint2 meta = a.blockMeta[b];
         const float* inv = a.blockInv + meta.x;
         const uint32_t* loc = a.blkLocal + (size_t)b * 32;
         const int tri = lane * (lane + 1) / 2;
-        for (int j = sub; j < (int)meta.y; j += SPLIT) {
+        for (int j = 0; j < (int)meta.y; ++j) {
           const float w = __ldg(inv + (j < lane ? tri + j : j * (j + 1) / 2 + lane));
           const float4 rj = sR[loc[j]];
           z[0] = fmaf(w, rj.x, z[0]); z[1] = fmaf(w, rj.y, z[1]); z[2] = fmaf(w, rj.z, z[2]);
@@ -468,13 +424,9 @@ __global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEA
     float zz[RPT][3];
 #pragma unroll
     for (int k = 0; k < RPT; ++k) {
-      const uint32_t l = (uint32_t)rt + (uint32_t)k * ROWS;
-      const bool act = l < m;
-      if (SPLIT == 1 && !act) continue;
-      zz[k][0] = zz[k][1] = zz[k][2] = 0.0f;
-      if (act) precond(k, zz[k]);
-      splitSum3<SPLIT>(zz[k]);
-      if (!act || sub != 0) continue;
+      const uint32_t l = (uint32_t)tid + (uint32_t)k * TEAM;
+      if (l >= m) continue;
+      precond(k, zz[k]);
       const float4 r = sR[l];
       red9[0] += r.x * zz[k][0]; red9[1] += r.y * zz[k][1]; red9[2] += r.z * zz[k][2];
       red9[3] += r.x * r.x; red9[4] += r.y * r.y; red9[5] += r.z * r.z;
@@ -484,32 +436,24 @@ __global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEA
     float rz[3] = {red9[0], red9[1], red9[2]};
     float rr[3] = {red9[3], red9[4], red9[5]};
     const float bb[3] = {red9[6], red9[7], red9[8]};
-    auto converged = [&]() {
-      return rr[0] <= a.tol2 * bb[0] + 1e-36f && rr[1] <= a.tol2 * bb[1] + 1e-36f && rr[2] <= a.tol2 * bb[2] + 1e-36f;
-    };
-    teamSync<TEAM>();  // p visible
+    __syncthreads();  // p visible
     uint32_t iters = 0;
-    bool conv = converged();
+    bool conv = converged3(rr, bb, a.tol2);
     while (!conv && iters < a.maxIter) {
       float ap[RPT][3];
       float pap[3] = {0.0f, 0.0f, 0.0f};
 #pragma unroll
       for (int k = 0; k < RPT; ++k) {
-        const uint32_t l = (uint32_t)rt + (uint32_t)k * ROWS;
+        const uint32_t l = (uint32_t)tid + (uint32_t)k * TEAM;
         ap[k][0] = ap[k][1] = ap[k][2] = 0.0f;
-        const bool act = l < m;
-        if (SPLIT == 1 && !act) continue;
-        if (act) {
-          const uint32_t e1 = rs[k] + rn[k];
+        if (l >= m) continue;
+        const uint32_t e1 = rs[k] + rn[k];
 #pragma unroll 4
-          for (uint32_t e = rs[k] + sub; e < e1; e += SPLIT) {
-            const float v = mv[e];
-            const float4 pv = sP[mc[e]];
-            ap[k][0] = fmaf(v, pv.x, ap[k][0]); ap[k][1] = fmaf(v, pv.y, ap[k][1]); ap[k][2] = fmaf(v, pv.z, ap[k][2]);
-          }
+        for (uint32_t e = rs[k]; e < e1; ++e) {
+          const float v = mv[e];
+          const float4 pv = sP[mc[e]];
+          ap[k][0] = fmaf(v, pv.x, ap[k][0]); ap[k][1] = fmaf(v, pv.y, ap[k][1]); ap[k][2] = fmaf(v, pv.z, ap[k][2]);
         }
-        splitSum3<SPLIT>(ap[k]);
-        if (!act || sub != 0) continue;
         const float4 pl = sP[l];
         ap[k][0] = fmaf(cdg[k], pl.x, ap[k][0]); ap[k][1] = fmaf(cdg[k], pl.y, ap[k][1]); ap[k][2] = fmaf(cdg[k], pl.z, ap[k][2]);
         pap[0] += pl.x * ap[k][0]; pap[1] += pl.y * ap[k][1]; pap[2] += pl.z * ap[k][2];
@@ -521,25 +465,21 @@ __global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEA
       float rl[RPT][3];
 #pragma unroll
       for (int k = 0; k < RPT; ++k) {
-        const uint32_t l = (uint32_t)rt + (uint32_t)k * ROWS;
-        if (l >= m || sub != 0) continue;
+        const uint32_t l = (uint32_t)tid + (uint32_t)k * TEAM;
+        if (l >= m) continue;
         const float4 pl = sP[l];
         dl[k][0] = fmaf(alpha[0], pl.x, dl[k][0]); dl[k][1] = fmaf(alpha[1], pl.y, dl[k][1]); dl[k][2] = fmaf(alpha[2], pl.z, dl[k][2]);
         const float4 r = sR[l];
         rl[k][0] = fmaf(-alpha[0], ap[k][0], r.x); rl[k][1] = fmaf(-alpha[1], ap[k][1], r.y); rl[k][2] = fmaf(-alpha[2], ap[k][2], r.z);
         sR[l] = make_float4(rl[k][0], rl[k][1], rl[k][2], 0.0f);
       }
-      teamSync<TEAM>();  // r visible
+      __syncthreads();  // r visible
       float red6[6] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
 #pragma unroll
       for (int k = 0; k < RPT; ++k) {
-        const uint32_t l = (uint32_t)rt + (uint32_t)k * ROWS;
-        const bool act = l < m;
-        if (SPLIT == 1 && !act) continue;
-        zz[k][0] = zz[k][1] = zz[k][2] = 0.0f;
-        if (act) precond(k, zz[k]);
-        splitSum3<SPLIT>(zz[k]);
-        if (!act || sub != 0) continue;
+        const uint32_t l = (uint32_t)tid + (uint32_t)k * TEAM;
+        if (l >= m) continue;
+        precond(k, zz[k]);
         red6[0] += rl[k][0] * zz[k][0]; red6[1] += rl[k][1] * zz[k][1]; red6[2] += rl[k][2] * zz[k][2];
         red6[3] += rl[k][0] * rl[k][0]; red6[4] += rl[k][1] * rl[k][1]; red6[5] += rl[k][2] * rl[k][2];
       }
@@ -548,38 +488,31 @@ __global__ void __launch_bounds__(TEAM == 32 ? 256 : TEAM, TEAM == 32 ? 3 : (TEA
 #pragma unroll
       for (int c = 0; c < 3; ++c) { beta[c] = rz[c] > 0.0f ? red6[c] / rz[c] : 0.0f; rz[c] = red6[c]; rr[c] = red6[3 + c]; }
       ++iters;
-      conv = converged();
+      conv = converged3(rr, bb, a.tol2);
       if (conv) break;
 #pragma unroll
       for (int k = 0; k < RPT; ++k) {
-        const uint32_t l = (uint32_t)rt + (uint32_t)k * ROWS;
-        if (l >= m || sub != 0) continue;
+        const uint32_t l = (uint32_t)tid + (uint32_t)k * TEAM;
+        if (l >= m) continue;
         const float4 pl = sP[l];
         sP[l] = make_float4(fmaf(beta[0], pl.x, zz[k][0]), fmaf(beta[1], pl.y, zz[k][1]), fmaf(beta[2], pl.z, zz[k][2]), 0.0f);
       }
-      teamSync<TEAM>();  // p visible
+      __syncthreads();  // p visible
     }
 #pragma unroll
     for (int k = 0; k < RPT; ++k) {
-      const uint32_t l = (uint32_t)rt + (uint32_t)k * ROWS;
-      if (l >= m || sub != 0) continue;
+      const uint32_t l = (uint32_t)tid + (uint32_t)k * TEAM;
+      if (l >= m) continue;
       float4 xv = a.x[gid[k]];
       xv.x += dl[k][0]; xv.y += dl[k][1]; xv.z += dl[k][2];
       a.x[gid[k]] = xv;
     }
     if (tid == 0) {
-      atomicMax(a.stats, iters);
-      atomicAdd(a.stats + 1, iters * ((m + 31u) >> 5));
-      if (!conv) {
-        float rel = 0.0f;
-        for (int c = 0; c < 3; ++c) if (bb[c] > 0.0f) rel = fmaxf(rel, rr[c] / bb[c]);
-        atomicAdd(a.stats + 2, 1u);
-        atomicMax(a.stats + 3, __float_as_uint(sqrtf(rel)));
-      }
+      recordSolve(a.stats, iters, m, conv, rr, bb);
       if (a.trace)
         a.trace[(size_t)tier * a.listStride + wi] = make_uint4(m, iters, (uint32_t)(clock64() - t0), a.nnzOff[s0 + m] - z0);
     }
-    teamSync<TEAM>();  // the team's shared memory is restaged for its next island
+    __syncthreads();  // the CTA's shared memory is restaged for its next island
   }
 }
 
@@ -663,17 +596,17 @@ __global__ void __launch_bounds__(256, 4) k_island_direct(IslandArgs a, int tier
     }
     float r0 = 0.0f, r1 = 0.0f, r2 = 0.0f;
     if (act) { r0 = (float)((double)bi.x - y0); r1 = (float)((double)bi.y - y1); r2 = (float)((double)bi.z - y2); }
-    const float bb0 = warpSum(bi.x * bi.x), bb1 = warpSum(bi.y * bi.y), bb2 = warpSum(bi.z * bi.z);
+    const float bb[3] = {warpSum(bi.x * bi.x), warpSum(bi.y * bi.y), warpSum(bi.z * bi.z)};
     float d0 = 0.0f, d1 = 0.0f, d2 = 0.0f;
     uint32_t iters = 0;
     bool conv = false;
-    float rr0, rr1, rr2;
+    float rr[3];
     asm volatile("cp.async.wait_group 0;\n" ::: "memory");
     __syncwarp();
     const float* inv = &sInv[warp][0];
     while (true) {
-      rr0 = warpSum(r0 * r0); rr1 = warpSum(r1 * r1); rr2 = warpSum(r2 * r2);
-      conv = rr0 <= a.tol2 * bb0 + 1e-36f && rr1 <= a.tol2 * bb1 + 1e-36f && rr2 <= a.tol2 * bb2 + 1e-36f;
+      rr[0] = warpSum(r0 * r0); rr[1] = warpSum(r1 * r1); rr[2] = warpSum(r2 * r2);
+      conv = converged3(rr, bb, a.tol2);
       if (conv || iters >= a.maxIter) break;
       // z = Minv r: lane with block lane bl owns row bl of the packed lower triangle
       float z0 = 0.0f, z1 = 0.0f, z2 = 0.0f;
@@ -705,16 +638,7 @@ __global__ void __launch_bounds__(256, 4) k_island_direct(IslandArgs a, int tier
       a.x[g] = xi;
     }
     if (lane == 0) {
-      atomicMax(a.stats, iters);
-      atomicAdd(a.stats + 1, iters);
-      if (!conv) {
-        float rel = 0.0f;
-        if (bb0 > 0.0f) rel = fmaxf(rel, rr0 / bb0);
-        if (bb1 > 0.0f) rel = fmaxf(rel, rr1 / bb1);
-        if (bb2 > 0.0f) rel = fmaxf(rel, rr2 / bb2);
-        atomicAdd(a.stats + 2, 1u);
-        atomicMax(a.stats + 3, __float_as_uint(sqrtf(rel)));
-      }
+      recordSolve(a.stats, iters, m, conv, rr, bb);
       if (a.trace) a.trace[(size_t)tier * a.listStride + wi] = make_uint4(m, iters, 0u, 0u);
     }
     __syncwarp();   // sInv / sLaneOf of this warp are rewritten for its next island
@@ -902,7 +826,7 @@ __global__ void __launch_bounds__(N, N <= 128 ? 8 : 5) k_island_dense(IslandArgs
     while (true) {
       rr[0] = r0 * r0; rr[1] = r1 * r1; rr[2] = r2 * r2;
       denseSum3<N / 32>(rr, sRed, phase, tid);
-      conv = rr[0] <= a.tol2 * bb[0] + 1e-36f && rr[1] <= a.tol2 * bb[1] + 1e-36f && rr[2] <= a.tol2 * bb[2] + 1e-36f;
+      conv = converged3(rr, bb, a.tol2);
       if (conv || iters >= a.maxIter) break;
       sV[tid] = make_float4(r0, r1, r2, 0.0f);
       __syncthreads();
@@ -956,14 +880,7 @@ __global__ void __launch_bounds__(N, N <= 128 ? 8 : 5) k_island_dense(IslandArgs
       a.x[g] = xi;
     }
     if (tid == 0) {
-      atomicMax(a.stats, iters);
-      atomicAdd(a.stats + 1, iters * ((m + 31u) >> 5));
-      if (!conv) {
-        float rel = 0.0f;
-        for (int c = 0; c < 3; ++c) if (bb[c] > 0.0f) rel = fmaxf(rel, rr[c] / bb[c]);
-        atomicAdd(a.stats + 2, 1u);
-        atomicMax(a.stats + 3, __float_as_uint(sqrtf(rel)));
-      }
+      recordSolve(a.stats, iters, m, conv, rr, bb);
       if (a.trace) a.trace[(size_t)slot * a.listStride + wi] = make_uint4(m, iters, (uint32_t)(clock64() - t0), a.nnzOff[s0 + m] - desc.w);
     }
     __syncthreads();   // sV / sRed are reused by the CTA's next island
@@ -1054,12 +971,9 @@ __global__ void __launch_bounds__(kBigTeam) k_island_pcg_big(IslandArgs a, uint3
     float rz[3] = {red9[0], red9[1], red9[2]};
     float rr[3] = {red9[3], red9[4], red9[5]};
     const float bb[3] = {red9[6], red9[7], red9[8]};
-    auto converged = [&]() {
-      return rr[0] <= a.tol2 * bb[0] + 1e-36f && rr[1] <= a.tol2 * bb[1] + 1e-36f && rr[2] <= a.tol2 * bb[2] + 1e-36f;
-    };
     __syncthreads();
     uint32_t iters = 0;
-    bool conv = converged();
+    bool conv = converged3(rr, bb, a.tol2);
     while (!conv && iters < a.maxIter) {
       float pap[3] = {0.0f, 0.0f, 0.0f};
       for (uint32_t l = (uint32_t)tid; l < m; l += kBigTeam) {
@@ -1101,7 +1015,7 @@ __global__ void __launch_bounds__(kBigTeam) k_island_pcg_big(IslandArgs a, uint3
 #pragma unroll
       for (int c = 0; c < 3; ++c) { beta[c] = rz[c] > 0.0f ? red6[c] / rz[c] : 0.0f; rz[c] = red6[c]; rr[c] = red6[3 + c]; }
       ++iters;
-      conv = converged();
+      conv = converged3(rr, bb, a.tol2);
       if (conv) break;
       for (uint32_t l = (uint32_t)tid; l < m; l += kBigTeam) {
         const float4 pl = sP[l], z = a.zScratch[s0 + l];
@@ -1116,32 +1030,23 @@ __global__ void __launch_bounds__(kBigTeam) k_island_pcg_big(IslandArgs a, uint3
       xv.x += d.x; xv.y += d.y; xv.z += d.z;
       a.x[g] = xv;
     }
-    if (tid == 0) {
-      atomicMax(a.stats, iters);
-      atomicAdd(a.stats + 1, iters * ((m + 31u) >> 5));
-      if (!conv) {
-        float rel = 0.0f;
-        for (int c = 0; c < 3; ++c) if (bb[c] > 0.0f) rel = fmaxf(rel, rr[c] / bb[c]);
-        atomicAdd(a.stats + 2, 1u);
-        atomicMax(a.stats + 3, __float_as_uint(sqrtf(rel)));
-      }
-    }
+    if (tid == 0) recordSolve(a.stats, iters, m, conv, rr, bb);
     __syncthreads();
   }
 }
 
 // ------------------------------------------------------------------------------------------------- host -----
 namespace {
-struct TierConfig { int team, rpt; bool matSmem; IslandCaps caps; int ctasPerSm; };
+struct TierConfig { int team, rpt; IslandCaps caps; };
 // caps: nodes, matrix entries, inverse floats, blocks resident in shared memory
 const TierConfig kTiers[kIslandSlots] = {
-    {32, 1, true, {32u, 640u, 576u, 4u}, 3},
-    {320, 2, true, {640u, 6656u, 9216u, 96u}, 2},
-    {512, 2, true, {1024u, 12288u, 17408u, 192u}, 1},
-    {1024, 0, false, {7168u, 0u, 0u, 0u}, 1},  // k_island_pcg_big
-    {128, 2, true, {256u, 2816u, 3456u, 32u}, 5},  // kSmallCtaSlot: 43 KB of shared memory
-    {128, 1, false, {kDenseMax, 0u, 0u, 0u}, 8},   // kDenseSlot: k_island_invert<128> + k_island_dense<128>
-    {192, 1, false, {kDenseMax2, 0u, 0u, 0u}, 5},  // kDenseSlot2: the same with N = 192
+    {32, 1, {32u, 640u, 576u, 4u}},         // k_island_direct
+    {320, 2, {640u, 6656u, 9216u, 96u}},
+    {512, 2, {1024u, 12288u, 17408u, 192u}},
+    {1024, 0, {7168u, 0u, 0u, 0u}},         // k_island_pcg_big
+    {128, 2, {256u, 2816u, 3456u, 32u}},    // kSmallCtaSlot: 43 KB of shared memory
+    {128, 1, {kDenseMax, 0u, 0u, 0u}},      // kDenseSlot: k_island_invert<128> + k_island_dense<128>
+    {192, 1, {kDenseMax2, 0u, 0u, 0u}},     // kDenseSlot2: the same with N = 192
 };
 // Test hook: PIES_B200_ISLAND_MAXBLOCKS=k shrinks the shared-memory block tables of the CTA tiers to k entries, so islands
 // with more preconditioner blocks exercise the from-global-memory path of the block-Jacobi apply.
@@ -1151,18 +1056,13 @@ IslandCaps tierCaps(int t) {
   if (forced > 0 && t >= 1 && c.maxBlocks) c.maxBlocks = std::min<uint32_t>(c.maxBlocks, (uint32_t)forced);
   return c;
 }
-IslandLayout tierLayout(int t) { return islandLayout(kTiers[t].caps, kTiers[t].team, kTiers[t].matSmem); }
-size_t tierSmem(int t) { return (size_t)tierLayout(t).total * (kTiers[t].team == 32 ? 8 : 1); }
-
-// t: whose team size, shared-memory layout and capacities; list: which island list (the same unless a list is handed to
-// a larger team)
+// k_island_pcg: t: whose team size, shared-memory layout and capacities; list: which island list (the same unless a list
+// is handed to a larger team)
 template <typename K>
-void launchTier(K kernel, int t, int grid, cudaStream_t s, const IslandArgs& a, int list = -1, int teamThreads = 0,
-                size_t smemAtLeast = 0) {
-  const size_t smem = std::max(tierSmem(t), smemAtLeast);
-  cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  const int threads = teamThreads ? teamThreads : (kTiers[t].team == 32 ? 256 : kTiers[t].team);
-  kernel<<<grid, threads, smem, s>>>(a, tierLayout(t), tierCaps(t), list < 0 ? t : list);
+void launchTier(K kernel, int t, int grid, cudaStream_t s, const IslandArgs& a, int list = -1) {
+  const IslandLayout L = islandLayout(kTiers[t].caps);
+  cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
+  kernel<<<grid, kTiers[t].team, L.total, s>>>(a, L, tierCaps(t), list < 0 ? t : list);
 }
 }  // namespace
 
@@ -1330,21 +1230,15 @@ int launchIslandSolve(IslandWork& w, cudaStream_t s, const CsrMatrix& S, const C
     k_island_pcg_big<<<(int)std::min<uint32_t>(w.tierCount[3], kNumSMs), kBigTeam, smem, nextStream()>>>(a, maxNodes, 3);
     ++L;
   }
-  if (w.tierCount[2]) { launchTier(k_island_pcg<512, 2, true>, 2, (int)std::min<uint32_t>(w.tierCount[2], kNumSMs), nextStream(), a); ++L; }
-  if (w.tierCount[1]) { launchTier(k_island_pcg<320, 2, true>, 1, (int)std::min<uint32_t>(w.tierCount[1], 2 * kNumSMs), nextStream(), a); ++L; }
+  if (w.tierCount[2]) { launchTier(k_island_pcg<512, 2>, 2, (int)std::min<uint32_t>(w.tierCount[2], kNumSMs), nextStream(), a); ++L; }
+  if (w.tierCount[1]) { launchTier(k_island_pcg<320, 2>, 1, (int)std::min<uint32_t>(w.tierCount[1], 2 * kNumSMs), nextStream(), a); ++L; }
   if (w.tierCount[kSmallCtaSlot]) {
     // A short list is latency bound (the solve waits for its slowest island, one warp per scheduler has nothing to hide
     // a dependent shared-memory load behind): the 320-thread team gives every row its own thread.  A long list is
     // throughput bound: five 128-thread CTAs per SM.
     const uint32_t ns = w.tierCount[kSmallCtaSlot];
-    // (measured, r02v/r02w: sharing a row between four lanes of a 1024-thread CTA is NOT faster — 10.8 k clocks per
-    // iteration against 8.9 k; the extra shuffles and reductions saturate the same shared-memory / shuffle pipe.  The
-    // variant stays reachable for experiments.)
-    static const bool split = std::getenv("PIES_B200_SPLIT_ROWS") != nullptr;
-    if (ns <= (uint32_t)kNumSMs && split)
-      launchTier(k_island_pcg<1024, 1, true, 4>, 1, (int)ns, nextStream(), a, kSmallCtaSlot, 1024);
-    else if (ns <= 2u * kNumSMs) launchTier(k_island_pcg<320, 2, true>, 1, (int)ns, nextStream(), a, kSmallCtaSlot);
-    else launchTier(k_island_pcg<128, 2, true>, kSmallCtaSlot, (int)std::min<uint32_t>(ns, 5 * kNumSMs), nextStream(), a);
+    if (ns <= 2u * kNumSMs) launchTier(k_island_pcg<320, 2>, 1, (int)ns, nextStream(), a, kSmallCtaSlot);
+    else launchTier(k_island_pcg<128, 2>, kSmallCtaSlot, (int)std::min<uint32_t>(ns, 5 * kNumSMs), nextStream(), a);
     ++L;
   }
   if (w.tierCount[kDenseSlot2]) {
@@ -1356,10 +1250,7 @@ int launchIslandSolve(IslandWork& w, cudaStream_t s, const CsrMatrix& S, const C
     ++L;
   }
   if (w.tierCount[0]) {
-    cudaStream_t st0 = nextStream();
-    static const bool staged = std::getenv("PIES_B200_WARP_TIER_STAGED") != nullptr;   // A/B switch: the staged PCG variant
-    if (staged) launchTier(k_island_pcg<32, 1, true>, 0, (int)std::min<uint32_t>((w.tierCount[0] + 7) / 8, 3 * kNumSMs), st0, a);
-    else k_island_direct<<<(int)std::min<uint32_t>((w.tierCount[0] + 7) / 8, 4 * kNumSMs), 256, 0, st0>>>(a, 0);
+    k_island_direct<<<(int)std::min<uint32_t>((w.tierCount[0] + 7) / 8, 4 * kNumSMs), 256, 0, nextStream()>>>(a, 0);
     ++L;
   }
   for (int k = 0; k < used; ++k) { cudaEventRecord(w.join[k], w.aux[k]); cudaStreamWaitEvent(s, w.join[k], 0); }
@@ -1382,11 +1273,9 @@ void preloadIslandKernels() {
   cudaFuncGetAttributes(&a, k_isl_starts);
   cudaFuncGetAttributes(&a, k_isl_nodes);
   cudaFuncGetAttributes(&a, k_isl_classify);
-  cudaFuncGetAttributes(&a, k_island_pcg<32, 1, true>);
-  cudaFuncGetAttributes(&a, k_island_pcg<320, 2, true>);
-  cudaFuncGetAttributes(&a, k_island_pcg<128, 2, true>);
-  cudaFuncGetAttributes(&a, k_island_pcg<1024, 1, true, 4>);
-  cudaFuncGetAttributes(&a, k_island_pcg<512, 2, true>);
+  cudaFuncGetAttributes(&a, k_island_pcg<320, 2>);
+  cudaFuncGetAttributes(&a, k_island_pcg<128, 2>);
+  cudaFuncGetAttributes(&a, k_island_pcg<512, 2>);
   cudaFuncGetAttributes(&a, k_island_pcg_big);
   cudaFuncGetAttributes(&a, k_island_direct);
   cudaFuncGetAttributes(&a, k_island_invert<(int)kDenseMax>);

@@ -1,4 +1,4 @@
-// islands.h — per-substep islands of the global solve and the island-local PCG (islands.cu).
+// islands.h — per-substep islands of the global solve and their island-local solves (islands.cu).
 #pragma once
 
 #include "engine.h"
@@ -7,8 +7,9 @@ namespace pies {
 
 // Tiers of the island-local solve.  An island is a connected component of S + C_t (static bodies joined by this
 // substep's contacts); the system matrix is block diagonal over islands, so every island is an independent solve.
-//   tier 0: one warp per island (<= 32 nodes in a single preconditioner block: every free body of the S3 stack)
-//   tier 1: one 320-thread CTA, matrix + block inverses + r, p resident in shared memory, two CTAs per SM
+//   tier 0: one warp per island (<= 32 nodes in a single preconditioner block: every free body of the S3 stack),
+//           iterative refinement with the block's exact inverse
+//   tier 1: one 320-thread CTA running CG, matrix + block inverses + r, p resident in shared memory, two CTAs per SM
 //   tier 2: one 512-thread CTA, the same with the whole shared memory of an SM
 //   tier 3: one 1024-thread CTA, r and p in shared memory, the island's matrix re-indexed in a global scratch copy
 //           (L2 resident: one CTA re-reads a few hundred KB per iteration)

@@ -414,10 +414,10 @@ def test_island_block_table_overflow_path(pb, monkeypatch, tmp_path):
     assert np.abs(a.positions - b).max() <= 1e-6 * bbox_diag(b)   # same arithmetic from another memory space
 
 
-@pytest.mark.parametrize("switch", ["PIES_B200_NO_DENSE", "PIES_B200_NO_DENSE2", "PIES_B200_NO_DENSE,PIES_B200_NO_SMALL_CTA", "PIES_B200_WARP_TIER_STAGED",
-                                    "PIES_B200_SPLIT_ROWS", "PIES_B200_NO_CELL_TABLE"])
+@pytest.mark.parametrize("switch", ["PIES_B200_NO_DENSE", "PIES_B200_NO_DENSE2", "PIES_B200_NO_DENSE,PIES_B200_NO_SMALL_CTA",
+                                    "PIES_B200_NO_CELL_TABLE"])
 def test_island_list_switches_agree(pb, switch, tmp_path):
-    """The A/B switches (no dense-inverse list, no 128-thread list, staged warp tier, rows shared by four lanes, radix-sorted cell table) route the same
+    """The A/B switches (no dense-inverse list, no 128-thread list, radix-sorted cell table) route the same
     work through the other kernels; all of them solve to the same tolerance, so the trajectories agree like the
     island / grid-wide pair above (compared while the contact counts agree)."""
     import subprocess, sys, os
