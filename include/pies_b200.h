@@ -307,6 +307,21 @@ int pies_b200_probe_sort_pairs(uint64_t n, uint64_t* keys, uint32_t* vals, int k
 int pies_b200_probe_sell(uint32_t n, const int32_t* rowPtr, const int32_t* col, const float* val, uint32_t* sellPtr,
                          uint32_t* sellRow, int32_t* sellCol, float* sellVal, uint64_t* paddedNnz);
 
+/* Host only: the closed segments of the fused local step + RHS (one CTA per segment, see DESIGN.md section 4) of a
+ * scene built from nCmds commands of 8 floats (kind, tx, ty, tz, a, b, c, d), t = translation:
+ *   kind 0: createTetBox(t, scale a, v0 0, w b, mass c, not hinged)
+ *   kind 1: createSheet(t, scale a, mass b, k c)
+ *   kind 2: createShapeMatchingBox(t, a x b x c particles, scale d, v0 0, w 1000)
+ *   kind 3: addTetMeshVolume of meshPoints + t and meshTets (no triangles), density 1, strain w 1000 in [0.8, 1],
+ *           volume w 1000 in [1, 1]
+ * sizes[0..6] = nodes, gather-list entries, fused tet elements, segments, elements outside segments, nodes outside
+ * segments, first tet contribution slot.  The arrays may be null (first call: sizes only); otherwise incPtr (nodes + 1),
+ * inc and segSlot (entries), elemIds (4 per element), segs (4 per segment: n0, n1, e0, e1), restElems, restNodes. */
+int pies_b200_probe_segments(uint32_t nCmds, const float* cmds, uint32_t nMeshPoints, const float* meshPoints,
+                             uint32_t nMeshTets, const uint32_t* meshTets, uint64_t* sizes, int32_t* incPtr, uint32_t* inc,
+                             uint16_t* segSlot, uint32_t* elemIds, uint32_t* segs, uint32_t* restElems,
+                             uint32_t* restNodes);
+
 #ifdef __cplusplus
 }
 #endif

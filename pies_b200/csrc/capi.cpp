@@ -623,3 +623,42 @@ extern "C" int pies_b200_probe_sell(uint32_t n, const int32_t* rowPtr, const int
     return PIES_B200_EINVAL;
   }
 }
+
+extern "C" int pies_b200_probe_segments(uint32_t nCmds, const float* cmds, uint32_t nMeshPoints, const float* meshPoints,
+                                        uint32_t nMeshTets, const uint32_t* meshTets, uint64_t* sizes, int32_t* incPtr,
+                                        uint32_t* inc, uint16_t* segSlot, uint32_t* elemIds, uint32_t* segs,
+                                        uint32_t* restElems, uint32_t* restNodes) {
+  if (!sizes || (nCmds && !cmds)) return PIES_B200_EINVAL;
+  try {
+    pies::HostScene sc;
+    const float zero[3] = {0.0f, 0.0f, 0.0f};
+    std::vector<float> pts;
+    for (uint32_t c = 0; c < nCmds; ++c) {
+      const float* m = cmds + 8ull * c;
+      const float* t = m + 1;
+      switch ((int)m[0]) {
+        case 0: sc.createTetBox(t, m[4], zero, m[5], m[6], false); break;
+        case 1: sc.createSheet(t, m[4], m[5], m[6]); break;
+        case 2: sc.createShapeMatchingBox(t, (uint32_t)m[4], (uint32_t)m[5], (uint32_t)m[6], m[7], zero, 1000.0f); break;
+        case 3:
+          if (!meshPoints || !meshTets) return PIES_B200_EINVAL;
+          pts.assign(meshPoints, meshPoints + 3ull * nMeshPoints);
+          for (size_t i = 0; i < pts.size(); ++i) pts[i] += t[i % 3];
+          sc.addTetMeshVolume(nMeshPoints, pts.data(), nMeshTets, meshTets, 0, nullptr, zero, 1.0f, 1000.0f, 0.8f, 1.0f,
+                              1000.0f, 1.0f, 1.0f);
+          break;
+        default: return PIES_B200_EINVAL;
+      }
+    }
+    pies::HostSystem y;
+    pies::buildSystem(sc, 1.0f / 60.0f, y, 1);
+    const uint64_t sz[7] = {y.n, y.inc.size(), y.nElems, y.segs.size() / 4, y.restElems.size(), y.restNodes.size(), y.baseTet};
+    std::memcpy(sizes, sz, sizeof(sz));
+    auto put = [](auto* dst, const auto& v) { if (dst) std::memcpy(dst, v.data(), v.size() * sizeof(v[0])); };
+    put(incPtr, y.incPtr); put(inc, y.inc); put(segSlot, y.segSlot); put(elemIds, y.elemIds); put(segs, y.segs);
+    put(restElems, y.restElems); put(restNodes, y.restNodes);
+    return PIES_B200_OK;
+  } catch (...) {
+    return PIES_B200_EINVAL;
+  }
+}

@@ -11,12 +11,11 @@
 #include "reblock.h"
 
 #include "common.cuh"
+#include "rhs.cuh"
 
 namespace pies {
 
 static inline int gridFor(uint64_t n, int threads) { return (int)((n + threads - 1) / threads); }
-
-constexpr float kFloorW = 10000.0f;  // StaticCollisionConstraint::w (CollisionConstraint.h:78)
 
 // ---- per-iteration projections (parallel, no ordering issue) ---------------------------------------
 // contribC[4u + slot] = copies * w * (A^T A p)_slot for distinct contact u, with p = current positions and
@@ -53,16 +52,18 @@ int launchContactProject(cudaStream_t s, const ContactLists& c, const float4* q,
 // The whole right-hand side in one pass when there are contacts: the constraint gather of k_gather_rhs (pd_kernels.cu),
 // then rhs_i += sum of the collision contributions (list order) + per floor duplicate w * projectedPosition
 // (Solver.cpp:337-349), in that order; the floor contacts' projectedPosition (the position with y < 0 -> 0) is written to
-// `snap` for the stabilisation sweeps.
-__global__ void __launch_bounds__(kThreads) k_gather_rhs_contacts(uint32_t n, const float4* __restrict__ msn,
+// `snap` for the stabilisation sweeps.  nodes: the nodes to assemble (null = 0 .. n-1).
+__global__ void __launch_bounds__(kThreads) k_gather_rhs_contacts(uint32_t n, const uint32_t* __restrict__ nodes,
+                                                                  const float4* __restrict__ msn,
                                                                   const int* __restrict__ incPtr,
                                                                   const uint32_t* __restrict__ inc,
                                                                   const float4* __restrict__ contrib, ContactLists c,
                                                                   const float4* __restrict__ contribC,
                                                                   const float4* __restrict__ q, float4* __restrict__ snap,
                                                                   float4* __restrict__ rhs) {
-  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const uint32_t i = nodes ? nodes[t] : t;
   float4 acc = ldStream(msn + i);
   {
     const int beg = incPtr[i], end = incPtr[i + 1];
@@ -80,28 +81,16 @@ __global__ void __launch_bounds__(kThreads) k_gather_rhs_contacts(uint32_t n, co
       acc.x += cv.x; acc.y += cv.y; acc.z += cv.z;
     }
   }
-  int beg = 0, end = 0;
-  if (c.nTri) { beg = c.incPtr[i]; end = c.incPtr[i + 1]; }
-  const uint32_t mult = c.nFloor ? c.floorMult[i] : 0u;
-  for (int k = beg; k < end; ++k) {
-    float4 v = contribC[c.inc[k]];
-    acc.x += v.x; acc.y += v.y; acc.z += v.z;
-  }
-  if (mult) {
-    float4 p = q[i];
-    if (p.y < 0.0f) p.y = 0.0f;
-    snap[i] = p;
-    for (uint32_t k = 0; k < mult; ++k) { acc.x += kFloorW * p.x; acc.y += kFloorW * p.y; acc.z += kFloorW * p.z; }
-  }
+  addContactTerms(acc, i, c, contribC, q, snap);
   acc.w = 0.0f;
   rhs[i] = acc;
 }
 
-int launchGatherRhsContacts(cudaStream_t s, uint32_t n, const float4* msn, const int* incPtr, const uint32_t* inc,
-                            const float4* contrib, const ContactLists& c, const float4* contribC, const float4* q,
-                            float4* snap, float4* rhs) {
+int launchGatherRhsContacts(cudaStream_t s, uint32_t n, const uint32_t* nodes, const float4* msn, const int* incPtr,
+                            const uint32_t* inc, const float4* contrib, const ContactLists& c, const float4* contribC,
+                            const float4* q, float4* snap, float4* rhs) {
   if (!n) return 0;
-  k_gather_rhs_contacts<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, msn, incPtr, inc, contrib, c, contribC, q, snap, rhs);
+  k_gather_rhs_contacts<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, nodes, msn, incPtr, inc, contrib, c, contribC, q, snap, rhs);
   return 1;
 }
 

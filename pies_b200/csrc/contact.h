@@ -60,9 +60,10 @@ int prepareContactSweeps(ContactWork& w, cudaStream_t s, const ContactLists& c);
 int prepareClusterSweeps(ContactWork& w, cudaStream_t s, const ContactLists& c, const ClusterTables& t);
 // Per PD iteration: collision projections (local step) and their RHS contributions.
 int launchContactProject(cudaStream_t s, const ContactLists& c, const float4* q, float thickness, float4* contribC);
-int launchGatherRhsContacts(cudaStream_t s, uint32_t n, const float4* msn, const int* incPtr, const uint32_t* inc,
-                            const float4* contrib, const ContactLists& c, const float4* contribC, const float4* q,
-                            float4* snap, float4* rhs);
+// nodes: the n nodes to assemble (null = 0 .. n-1)
+int launchGatherRhsContacts(cudaStream_t s, uint32_t n, const uint32_t* nodes, const float4* msn, const int* incPtr,
+                            const uint32_t* inc, const float4* contrib, const ContactLists& c, const float4* contribC,
+                            const float4* q, float4* snap, float4* rhs);
 // End of substep: ordered stabilisation sweeps (list order per node, see contact.cu) and the friction pass.
 int launchStabilize(cudaStream_t s, ContactWork& w, const ContactLists& c, uint32_t n, float4* q, float4* prev,
                     const float4* snap, float thickness, uint32_t iterations);

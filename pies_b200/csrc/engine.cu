@@ -208,6 +208,8 @@ int ensureBuilt(PiesB200Solver* s) {
   PIES_CHECK(s, s->goalXform.upload(reinterpret_cast<const float*>(sc.goalXform.data()), sc.goalXform.size() * 16, st));
   sc.goalXformDirty = false;
   PIES_CHECK(s, uploadVec(s->incPtr, y.incPtr, st)); PIES_CHECK(s, uploadVec(s->inc, y.inc, st));
+  PIES_CHECK(s, uploadVec(s->segs, y.segs, st)); PIES_CHECK(s, uploadVec(s->segSlot, y.segSlot, st));
+  PIES_CHECK(s, uploadVec(s->restElems, y.restElems, st)); PIES_CHECK(s, uploadVec(s->restNodes, y.restNodes, st));
   PIES_CHECK(s, uploadVec(s->rowPtr, y.rowPtr, st)); PIES_CHECK(s, uploadVec(s->col, y.col, st)); PIES_CHECK(s, uploadVec(s->val, y.val, st));
   PIES_CHECK(s, uploadVec(s->sellPtr, y.sellPtr, st)); PIES_CHECK(s, uploadVec(s->sellRow, y.sellRow, st));
   PIES_CHECK(s, uploadVec(s->sellCol, y.sellCol, st)); PIES_CHECK(s, uploadVec(s->sellVal, y.sellVal, st));
@@ -514,23 +516,37 @@ int pdIteration(PiesB200Solver* s) {
   const ContactLists& lists = c->lists;
   PdViews v = pdViews(s);
   float4* contribC = s->contact ? s->contact->contribC.p : nullptr;
-  timer.begin(kPhTetKernel);
-  s->launches += launchTetElems(st, v.te, s->q.p, s->contrib.p + y.baseTet);
-  timer.end();
+  const bool anyContact = lists.nTri || lists.nFloor;
+  // The fused local step + RHS (k_tet_rhs) covers the closed segments; the elements and nodes outside them take the
+  // two-kernel path.  A/B switch: PIES_B200_NO_FUSED_LOCAL sends everything through the two-kernel path.
+  static const bool noFused = std::getenv("PIES_B200_NO_FUSED_LOCAL") != nullptr;
+  const bool fused = !noFused && !y.segs.empty();
+  const TetSegments sg{s->segs.p, s->segSlot.p, fused ? (uint32_t)(y.segs.size() / 4) : 0u};
+  const uint32_t* tetList = fused ? s->restElems.p : nullptr;
+  const uint32_t* nodeList = fused ? s->restNodes.p : nullptr;
+  const uint32_t nTetList = fused ? (uint32_t)y.restElems.size() : y.nElems;
+  const uint32_t nNodeList = fused ? (uint32_t)y.restNodes.size() : n;
+  // the local span holds the tet span (msLocal is the whole local step + RHS)
   const int spLocal = timer.begin(kPhLocal);
+  s->launches += launchContactProject(st, lists, s->q.p, s->opt.collisionThickness, contribC);  // k_tet_rhs reads contribC
+  // the tet slot times the tet projections of both paths, with the RHS of the segments when fused
+  const int spTet = timer.begin(kPhTetKernel);
+  s->launches += launchTetRhs(st, v.te, sg, s->q.p, s->msn.p, s->incPtr.p, lists, contribC, s->snap.p, s->rhs.p);
+  s->launches += launchTetElems(st, v.te, tetList, nTetList, s->q.p, s->contrib.p + y.baseTet);
+  timer.end(spTet);
   s->launches += launchDistance(st, v.de, s->q.p, s->contrib.p + y.baseDist);
   s->launches += launchBend(st, v.be, s->q.p, s->contrib.p + y.baseBend);
   s->launches += launchShape(st, v.sh, s->shapeMat.p, s->shapeQinv.p, s->shapeQuat.p, s->shapeW.p, s->q.p, s->contrib.p + y.baseShape);
   s->launches += launchGoal(st, v.go, s->goalMat.p, s->goalXform.p, s->goalW.p, s->contrib.p + y.baseGoal);
-  const bool anyContact = lists.nTri || lists.nFloor;
-  s->launches += launchContactProject(st, lists, s->q.p, s->opt.collisionThickness, contribC);
-  const int spGather = timer.begin(kPhGatherKernel);
-  if (anyContact)   // constraints + collision + floor terms in one pass over the nodes (it also writes the floor snap)
-    s->launches += launchGatherRhsContacts(st, n, s->msn.p, s->incPtr.p, s->inc.p, s->contrib.p, lists, contribC, s->q.p,
-                                           s->snap.p, s->rhs.p);
-  else
-    s->launches += launchGatherRhs(st, n, s->msn.p, s->incPtr.p, s->inc.p, s->contrib.p, s->rhs.p);
-  timer.end(spGather);
+  if (nNodeList) {
+    const int spGather = timer.begin(kPhGatherKernel);
+    if (anyContact)   // constraints + collision + floor terms in one pass over the nodes (it also writes the floor snap)
+      s->launches += launchGatherRhsContacts(st, nNodeList, nodeList, s->msn.p, s->incPtr.p, s->inc.p, s->contrib.p, lists,
+                                             contribC, s->q.p, s->snap.p, s->rhs.p);
+    else
+      s->launches += launchGatherRhs(st, nNodeList, nodeList, s->msn.p, s->incPtr.p, s->inc.p, s->contrib.p, s->rhs.p);
+    timer.end(spGather);
+  }
   timer.end(spLocal);
 
   const int spGlobal = timer.begin(kPhGlobal);
@@ -657,7 +673,7 @@ int pdTickEnd(PiesB200Solver* s, bool refreshMirror) {
     float acc[kPhCount] = {};
     uint32_t cnt[kPhCount] = {};
     c->timer.resolve(acc, cnt);
-    s->stats.msOther = acc[kPhOther]; s->stats.msDetect = acc[kPhDetect]; s->stats.msLocal = acc[kPhLocal] + acc[kPhTetKernel];
+    s->stats.msOther = acc[kPhOther]; s->stats.msDetect = acc[kPhDetect]; s->stats.msLocal = acc[kPhLocal];
     s->stats.msGlobal = acc[kPhGlobal]; s->stats.msContact = acc[kPhContact];
     s->stats.msTetKernel = acc[kPhTetKernel]; s->stats.tetKernelLaunches = cnt[kPhTetKernel];
     s->stats.msSpmvKernel = acc[kPhSpmvKernel]; s->stats.spmvKernelLaunches = cnt[kPhSpmvKernel];

@@ -84,6 +84,7 @@ struct PiesB200Solver {
   pies::DevBuf<double> shapeMat, shapeQinv, shapeQuat;
   pies::DevBuf<float> shapeW, goalMat, goalXform, goalW;
   pies::DevBuf<int> incPtr; pies::DevBuf<uint32_t> inc;
+  pies::DevBuf<uint4> segs; pies::DevBuf<uint16_t> segSlot; pies::DevBuf<uint32_t> restElems, restNodes;  // HostSystem::segs
   pies::DevBuf<int> rowPtr, col; pies::DevBuf<float> val;
   pies::DevBuf<uint32_t> sellPtr, sellRow; pies::DevBuf<int> sellCol; pies::DevBuf<float> sellVal;
   pies::DevBuf<int> blockNodes; pies::DevBuf<float> blockInv;

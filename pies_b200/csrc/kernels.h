@@ -27,6 +27,17 @@ struct TetElems {
   uint32_t n = 0;
 };
 
+// Closed segments of the fused local step + RHS (k_tet_rhs; built by buildSegments, system.h): per segment the node
+// range [n0, n1) and the element range [e0, e1) that one CTA projects and assembles on chip.
+constexpr uint32_t kSegElems = 256;     // cap per segment: 4 float4 contributions per element in shared memory ...
+constexpr uint32_t kSegNodes = 256;     // ... and one staged float4 position per node (20 KB per CTA)
+constexpr int kTetRhsThreads = 128;     // CTA of k_tet_rhs (elements, then nodes, strided over the threads)
+struct TetSegments {
+  const uint4* segs = nullptr;          // (n0, n1, e0, e1)
+  const uint16_t* slot = nullptr;       // parallel to the gather list inc: 4 (e - e0) + k for the nodes of a segment
+  uint32_t n = 0;
+};
+
 struct DistanceElems { uint2* ids = nullptr; float2* restW = nullptr; uint32_t n = 0; };
 struct BendElems { uint4* ids = nullptr; float2* angleW = nullptr; uint32_t n = 0; };
 struct ClusterElems {  // shape- and goal-matching clusters (CSR over members)
@@ -70,15 +81,20 @@ struct ContactLists {
 
 // ------------------------------------------------------------- PD kernels ----
 int launchPredict(cudaStream_t s, uint32_t n, float4* q, const float4* vel, float4* msn, float h);
-int launchTetElems(cudaStream_t s, const TetElems& e, const float4* q, float4* contrib);
+// list: the n elements to project (null = 0 .. n-1)
+int launchTetElems(cudaStream_t s, const TetElems& e, const uint32_t* list, uint32_t n, const float4* q, float4* contrib);
 int launchDistance(cudaStream_t s, const DistanceElems& e, const float4* q, float4* contrib);
 int launchBend(cudaStream_t s, const BendElems& e, const float4* q, float4* contrib);
 int launchGoal(cudaStream_t s, const ClusterElems& c, const float* material /*3 per member*/,
                const float* xform /*16 per cluster*/, const float* w, float4* contrib);
 int launchShape(cudaStream_t s, const ClusterElems& c, const double* material, const double* qinv,
                 double* quat /*4 per cluster, state*/, const float* w, const float4* q, float4* contrib);
-int launchGatherRhs(cudaStream_t s, uint32_t n, const float4* msn, const int* incPtr, const uint32_t* inc,
-                    const float4* contrib, float4* rhs);
+// nodes: the n nodes to assemble (null = 0 .. n-1)
+int launchGatherRhs(cudaStream_t s, uint32_t n, const uint32_t* nodes, const float4* msn, const int* incPtr,
+                    const uint32_t* inc, const float4* contrib, float4* rhs);
+// Fused tet projections + RHS of every node of the segments (with the collision and floor terms of c when it has any).
+int launchTetRhs(cudaStream_t s, const TetElems& e, const TetSegments& sg, const float4* q, const float4* msn,
+                 const int* incPtr, const ContactLists& c, const float4* contribC, float4* snap, float4* rhs);
 int launchVelocityUpdate(cudaStream_t s, uint32_t n, const float4* q, float4* prev, float4* vel, float h,
                          float damping, float gravity);
 

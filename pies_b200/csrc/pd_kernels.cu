@@ -8,6 +8,7 @@
 // contribution has its own slot; a CSR gather sums them in a fixed order, which
 // makes the right-hand side run-to-run bit-stable).
 #include "kernels.h"
+#include "rhs.cuh"
 #include "svd3.cuh"
 
 namespace pies {
@@ -38,14 +39,13 @@ int launchPredict(cudaStream_t s, uint32_t n, float4* q, const float4* vel, floa
 // One thread per tet: gather 4 nodes, F = P Qinv, one SVD shared by both constraints,
 // contribution_i = (w_s Fhat_s + w_v Fhat_v) Qinv^T (columns for nodes 2..4; node 1 gets
 // minus their sum, i.e. w A^T B p with A = [0; Qinv^T D], B = I).
-__global__ void __launch_bounds__(128) k_tet_elems(TetElems e, const float4* __restrict__ q,
-                                                   float4* __restrict__ contrib) {
-  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= e.n) return;
+// The projection of element i, shared by k_tet_elems and k_tet_rhs; node(id) returns the position of node id.
+template <typename NodeFn>
+__device__ __forceinline__ void tetContribs(const TetElems& e, uint32_t i, NodeFn node, float4 (&out)[4]) {
   uint4 id = ldStream(e.ids + i);
   float4 qa = ldStream(e.qa + i), qb = ldStream(e.qb + i), pc = ldStream(e.pc + i), pd = ldStream(e.pd + i);
   float qinv[9] = {qa.x, qa.y, qa.z, qa.w, qb.x, qb.y, qb.z, qb.w, pc.x};
-  V3 x1 = v3(__ldg(q + id.x)), x2 = v3(__ldg(q + id.y)), x3 = v3(__ldg(q + id.z)), x4 = v3(__ldg(q + id.w));
+  V3 x1 = v3(node(id.x)), x2 = v3(node(id.y)), x3 = v3(node(id.z)), x4 = v3(node(id.w));
   M3 F = deformationGradient(x1, x2, x3, x4, qinv);
   M3 U, V;
   float sg[3];
@@ -86,13 +86,69 @@ __global__ void __launch_bounds__(128) k_tet_elems(TetElems e, const float4* __r
   V3 c0 = v3(T.m[0][0] * a0[0] + T.m[0][1] * a0[1] + T.m[0][2] * a0[2],
              T.m[1][0] * a0[0] + T.m[1][1] * a0[1] + T.m[1][2] * a0[2],
              T.m[2][0] * a0[0] + T.m[2][1] * a0[1] + T.m[2][2] * a0[2]);
-  float4* out = contrib + 4ull * i;
   out[0] = f4(c0, 0.0f); out[1] = f4(c[0], 0.0f); out[2] = f4(c[1], 0.0f); out[3] = f4(c[2], 0.0f);
 }
 
-int launchTetElems(cudaStream_t s, const TetElems& e, const float4* q, float4* contrib) {
-  if (!e.n) return 0;
-  k_tet_elems<<<gridFor(e.n, 128), 128, 0, s>>>(e, q, contrib);
+// list: the elements to project (null = 0 .. n-1)
+__global__ void __launch_bounds__(128) k_tet_elems(TetElems e, const uint32_t* __restrict__ list, uint32_t n,
+                                                   const float4* __restrict__ q, float4* __restrict__ contrib) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const uint32_t i = list ? list[t] : t;
+  float4 c[4];
+  tetContribs(e, i, [&](uint32_t id) { return __ldg(q + id); }, c);
+  float4* out = contrib + 4ull * i;
+  out[0] = c[0]; out[1] = c[1]; out[2] = c[2]; out[3] = c[3];
+}
+
+int launchTetElems(cudaStream_t s, const TetElems& e, const uint32_t* list, uint32_t n, const float4* q, float4* contrib) {
+  if (!n) return 0;
+  k_tet_elems<<<gridFor(n, 128), 128, 0, s>>>(e, list, n, q, contrib);
+  return 1;
+}
+
+// ---- fused local step + RHS over closed segments (HostSystem::segs) -------------------------------------
+// One CTA per segment.  Its nodes' positions are staged in shared memory; each thread projects elements exactly like
+// k_tet_elems and keeps their four contributions in shared memory; then each thread assembles nodes like
+// k_gather_rhs_contacts: msn, plus the contributions in the order of the global gather list (slot = the same list in
+// segment-local slots), plus the collision and floor terms.  The same code and the same sequence of float adds as the
+// two-kernel path, so the same bits, without the contributions' round trip through HBM and the inc gather.
+// Eight CTAs per SM (32 warps, 64 registers: a 52 B spill of loop state to L1) measured 75.0 us per iteration at S3 on a
+// B200, seven (72 registers) 77.3 us, six (78, no spill) 81.3 us; one 256-thread CTA per segment 93.6 us.
+__global__ void __launch_bounds__(kTetRhsThreads, 8) k_tet_rhs(TetElems e, TetSegments sg, const float4* __restrict__ q,
+                                                            const float4* __restrict__ msn, const int* __restrict__ incPtr,
+                                                            ContactLists c, const float4* __restrict__ contribC,
+                                                            float4* __restrict__ snap, float4* __restrict__ rhs) {
+  __shared__ float4 sQ[kSegNodes];
+  __shared__ float4 sC[4 * kSegElems];
+  const uint4 g = sg.segs[blockIdx.x];  // n0, n1, e0, e1
+  const uint32_t nN = g.y - g.x, nE = g.w - g.z;
+  for (uint32_t v = threadIdx.x; v < nN; v += kTetRhsThreads) sQ[v] = __ldg(q + g.x + v);
+  __syncthreads();
+  for (uint32_t t = threadIdx.x; t < nE; t += kTetRhsThreads) {
+    float4 cv[4];
+    tetContribs(e, g.z + t, [&](uint32_t id) { return sQ[id - g.x]; }, cv);
+    sC[4 * t] = cv[0]; sC[4 * t + 1] = cv[1]; sC[4 * t + 2] = cv[2]; sC[4 * t + 3] = cv[3];
+  }
+  __syncthreads();
+  for (uint32_t v = threadIdx.x; v < nN; v += kTetRhsThreads) {
+    const uint32_t i = g.x + v;
+    float4 acc = ldStream(msn + i);
+    const int beg = incPtr[i], end = incPtr[i + 1];
+    for (int k = beg; k < end; ++k) {
+      const float4 cv = sC[sg.slot[k]];
+      acc.x += cv.x; acc.y += cv.y; acc.z += cv.z;
+    }
+    addContactTerms(acc, i, c, contribC, q, snap);
+    acc.w = 0.0f;
+    rhs[i] = acc;
+  }
+}
+
+int launchTetRhs(cudaStream_t s, const TetElems& e, const TetSegments& sg, const float4* q, const float4* msn,
+                 const int* incPtr, const ContactLists& c, const float4* contribC, float4* snap, float4* rhs) {
+  if (!sg.n) return 0;
+  k_tet_rhs<<<sg.n, kTetRhsThreads, 0, s>>>(e, sg, q, msn, incPtr, c, contribC, snap, rhs);
   return 1;
 }
 
@@ -297,14 +353,16 @@ int launchShape(cudaStream_t s, const ClusterElems& c, const double* material, c
 
 // ---- RHS assembly: deterministic CSR gather (replaces Constraints.h:89-105 scatter-adds) ------------
 // rhs_i = Msn_h2_i + sum over the node's incidences, in the reference's type order
-// (position, distance, tet/volume, bend, shape, goal) then creation order.
-__global__ void __launch_bounds__(kThreads) k_gather_rhs(uint32_t n, const float4* __restrict__ msn,
+// (position, distance, tet/volume, bend, shape, goal) then creation order.  nodes: the nodes to assemble (null = 0 .. n-1).
+__global__ void __launch_bounds__(kThreads) k_gather_rhs(uint32_t n, const uint32_t* __restrict__ nodes,
+                                                         const float4* __restrict__ msn,
                                                          const int* __restrict__ incPtr,
                                                          const uint32_t* __restrict__ inc,
                                                          const float4* __restrict__ contrib,
                                                          float4* __restrict__ rhs) {
-  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const uint32_t i = nodes ? nodes[t] : t;
   float4 acc = ldStream(msn + i);
   int beg = incPtr[i], end = incPtr[i + 1];
   int k = beg;
@@ -324,10 +382,10 @@ __global__ void __launch_bounds__(kThreads) k_gather_rhs(uint32_t n, const float
   rhs[i] = acc;
 }
 
-int launchGatherRhs(cudaStream_t s, uint32_t n, const float4* msn, const int* incPtr, const uint32_t* inc,
-                    const float4* contrib, float4* rhs) {
+int launchGatherRhs(cudaStream_t s, uint32_t n, const uint32_t* nodes, const float4* msn, const int* incPtr,
+                    const uint32_t* inc, const float4* contrib, float4* rhs) {
   if (!n) return 0;
-  k_gather_rhs<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, msn, incPtr, inc, contrib, rhs);
+  k_gather_rhs<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, nodes, msn, incPtr, inc, contrib, rhs);
   return 1;
 }
 

@@ -97,6 +97,67 @@ void buildSell(uint32_t n, const int* rowPtr, const int* col, const float* val, 
   }
 }
 
+void buildSegments(HostSystem& y) {
+  y.segs.clear(); y.restElems.clear(); y.restNodes.clear();
+  y.segSlot.assign(y.inc.size(), 0);
+  const uint64_t tetEnd = y.baseTet + 4ull * y.nElems;
+  constexpr uint32_t kNone = 0xffffffffu;
+  uint32_t cur[4] = {0, 0, kNone, kNone};  // open segment: n0, n1, e0, e1 (e0 == kNone: no element yet)
+  bool open = false;
+  auto close = [&]() {
+    if (!open) return;
+    if (cur[2] == kNone) cur[2] = cur[3] = 0;
+    y.segs.insert(y.segs.end(), cur, cur + 4);
+    open = false;
+  };
+  for (uint32_t b = 0; b < y.nBodies; ++b) {
+    const uint32_t p0 = y.bodyPtr[b], cnt = y.bodyPtr[b + 1] - p0, a = y.bodyNodes[p0];
+    bool ok = y.bodyNodes[p0 + cnt - 1] - a + 1 == cnt && cnt <= kSegNodes;  // bodyNodes is ascending
+    uint32_t eLo = kNone, eHi = 0;
+    for (uint32_t i = a; ok && i < a + cnt; ++i)
+      for (int k = y.incPtr[i]; k < y.incPtr[i + 1]; ++k) {
+        const uint64_t slot = y.inc[k];
+        if (slot < y.baseTet || slot >= tetEnd) { ok = false; break; }
+        const uint32_t e = (uint32_t)((slot - y.baseTet) / 4);
+        eLo = std::min(eLo, e); eHi = std::max(eHi, e);
+      }
+    const bool hasElems = eLo != kNone;
+    ok = ok && (!hasElems || eHi - eLo + 1 <= kSegElems);
+    for (uint32_t e = eLo; ok && hasElems && e <= eHi; ++e)   // the range holds no element of another body
+      for (int k = 0; k < 4; ++k) {
+        const uint32_t v = y.elemIds[4ull * e + k];
+        if (v < a || v >= a + cnt) { ok = false; break; }
+      }
+    if (!ok) { close(); continue; }
+    const uint32_t nE = hasElems ? eHi + 1 - eLo : 0;
+    const uint32_t curE = cur[2] == kNone ? 0 : cur[3] - cur[2];
+    const bool joins = open && a == cur[1] && cur[1] - cur[0] + cnt <= kSegNodes &&
+                       curE + nE <= kSegElems && (!hasElems || cur[2] == kNone || eLo == cur[3]);
+    if (!joins) {
+      close();
+      cur[0] = cur[1] = a; cur[2] = cur[3] = kNone;
+      open = true;
+    }
+    cur[1] = a + cnt;
+    if (hasElems) {
+      if (cur[2] == kNone) cur[2] = eLo;
+      cur[3] = eHi + 1;
+    }
+  }
+  close();
+  std::vector<char> nodeIn(y.n, 0), elemIn(y.nElems, 0);
+  for (size_t s = 0; s < y.segs.size(); s += 4) {
+    const uint32_t n0 = y.segs[s], n1 = y.segs[s + 1], e0 = y.segs[s + 2], e1 = y.segs[s + 3];
+    for (uint32_t i = n0; i < n1; ++i) {
+      nodeIn[i] = 1;
+      for (int k = y.incPtr[i]; k < y.incPtr[i + 1]; ++k) y.segSlot[k] = (uint16_t)(y.inc[k] - y.baseTet - 4ull * e0);
+    }
+    for (uint32_t e = e0; e < e1; ++e) elemIn[e] = 1;
+  }
+  for (uint32_t i = 0; i < y.n; ++i) if (!nodeIn[i]) y.restNodes.push_back(i);
+  for (uint32_t e = 0; e < y.nElems; ++e) if (!elemIn[e]) y.restElems.push_back(e);
+}
+
 void buildSystem(const HostScene& sc, float h, HostSystem& out, unsigned threads) {
   out = HostSystem{};
   const uint32_t n = sc.nodeCount();
@@ -323,6 +384,7 @@ void buildSystem(const HostScene& sc, float h, HostSystem& out, unsigned threads
         out.colRank[k] = out.bodyOf[c] == out.bodyOf[r] ? out.rankInBody[c] : 0xffffffffu;
       }
   }
+  buildSegments(out);
   out.blockInv.assign((size_t)out.nBlocks * 1024, 0.0f);
   auto invertBlocks = [&](unsigned t) {
     std::vector<double> a(32 * 32), inv(32 * 32);

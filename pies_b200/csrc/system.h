@@ -4,6 +4,7 @@
 #include <cstdint>
 #include <vector>
 
+#include "kernels.h"
 #include "scene.h"
 
 namespace pies {
@@ -53,8 +54,21 @@ struct HostSystem {
   // outside the row's body (bend stencils); lets the island solver re-index a row without a gather per entry
   std::vector<uint32_t> colRank;
 
+  // Closed segments of the fused local step + RHS (k_tet_rhs, one CTA per segment).  A segment is a run of whole bodies
+  // whose nodes are one index range [n0, n1) and whose fused tet elements are one range [e0, e1), such that the elements
+  // reference only nodes of [n0, n1) and every incidence of those nodes is a tet slot of an element in [e0, e1) (no
+  // other constraint type touches them), and at most kSegElems elements and kSegNodes nodes (kernels.h).  Its
+  // contributions then never have to leave the CTA.  Bodies that break a condition keep the two-kernel path: their
+  // elements are listed in restElems, their nodes in restNodes (both ascending).
+  std::vector<uint32_t> segs;                 // 4 per segment: n0, n1, e0, e1
+  std::vector<uint16_t> segSlot;              // parallel to inc: 4 (e - e0) + k for an incidence of a segment node, else 0
+  std::vector<uint32_t> restElems, restNodes;
+
   uint64_t staticProjections = 0;             // per PD iteration, shape/goal count one per member
 };
+
+// Fills the segment fields of a HostSystem whose elements and gather lists are built.  O(n + incidences).
+void buildSegments(HostSystem& y);
 
 // Sliced-ELLPACK copy of a CSR matrix (layout described in HostSystem).  Host only.
 void buildSell(uint32_t n, const int* rowPtr, const int* col, const float* val, std::vector<uint32_t>& sellPtr,

@@ -149,6 +149,7 @@ _SIGNATURES = {
     "pies_b200_probe_node_range": (C.c_int, [C.c_uint32, _f32p, _f32p, C.c_float, _i64p, _u32p]),
     "pies_b200_probe_sort_pairs": (C.c_int, [C.c_uint64, _u64p, _u32p, C.c_int]),
     "pies_b200_probe_sell": (C.c_int, [C.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(C.c_uint64)]),
+    "pies_b200_probe_segments": (C.c_int, [C.c_uint32, _vp, C.c_uint32, _vp, C.c_uint32, _vp, _u64p] + [_vp] * 7),
 }
 
 _lib = None
@@ -612,3 +613,23 @@ def probe_sell(rowPtr, col, val):
     sc = np.zeros(padded.value, np.int32); sv = np.zeros(padded.value, np.float32)
     _ckp(lib().pies_b200_probe_sell(n, p(rp), p(c), p(v), p(sp), p(sr), p(sc), p(sv), C.byref(padded)))
     return sp, sr, sc, sv
+
+
+def probe_segments(cmds, mesh_points=None, mesh_tets=None):
+    """Host-only: the closed segments of the fused local step + RHS for a scene built from commands (rows of
+    kind, tx, ty, tz, a, b, c, d; see pies_b200_probe_segments), with the gather lists they were cut from."""
+    cm = np.ascontiguousarray(cmds, np.float32).reshape(-1, 8)
+    mp = None if mesh_points is None else np.ascontiguousarray(mesh_points, np.float32).reshape(-1, 3)
+    mt = None if mesh_tets is None else np.ascontiguousarray(mesh_tets, np.uint32).reshape(-1, 4)
+    p = lambda a: None if a is None else a.ctypes.data_as(_vp)
+    head = (len(cm), p(cm), 0 if mp is None else len(mp), p(mp), 0 if mt is None else len(mt), p(mt))
+    sizes = np.zeros(7, np.uint64)
+    _ckp(lib().pies_b200_probe_segments(*head, sizes, *([None] * 7)))
+    n, ninc, ne, ns, nre, nrn, base = (int(x) for x in sizes)
+    out = dict(incPtr=np.zeros(n + 1, np.int32), inc=np.zeros(ninc, np.uint32), segSlot=np.zeros(ninc, np.uint16),
+               elemIds=np.zeros((ne, 4), np.uint32), segs=np.zeros((ns, 4), np.uint32),
+               restElems=np.zeros(nre, np.uint32), restNodes=np.zeros(nrn, np.uint32))
+    keys = ("incPtr", "inc", "segSlot", "elemIds", "segs", "restElems", "restNodes")
+    _ckp(lib().pies_b200_probe_segments(*head, sizes, *(p(out[k]) for k in keys)))
+    out["baseTet"] = base
+    return out
