@@ -157,6 +157,44 @@ int pies_b200_set_render_state_dirty(PiesB200Solver* s, int dirty);
 int pies_b200_sim_failed(const PiesB200Solver* s);               /* the _simFailed latch, Solver.cpp:26-28,852-856 */
 int pies_b200_clear(PiesB200Solver* s);                          /* Solver::clear, Solver.cpp:488-507 */
 
+/* ---- [additive] static colliders: half-spaces, spheres and oriented solid boxes (DESIGN.md section 9).
+ *      The reference has no collision geometry but the floor; a host that wants a container, a ramp or an obstacle sets
+ *      them here.  Each collider k has a signed distance phi_k(x) (negative inside) and an outward normal n_k(x):
+ *        half-space: phi = n . (x - c), n normalised by the library;
+ *        sphere:     phi = |x - c| - r, n = (x - c) / |x - c| (n = +y at x = c);
+ *        box:        the box signed distance in its local frame; outside, n points from the closest surface point to x;
+ *                    inside, n is the normal of the nearest face (tie: lowest axis first, then the + side).
+ *      Colliders are static during a tick and evaluated in ascending index order everywhere.  The set may be replaced
+ *      between ticks (moving an obstacle rebuilds nothing).
+ *      PD: a node with phi_k(q) < collisionThickness at detection is in contact with k for the substep; every iteration
+ *      it is pulled towards q - min(phi_k(q), 0) n_k(q) with weight 1e4 (the floor's weight); after stabilisation it is
+ *      projected out of its colliders, and friction acts along each collider's tangent plane.  The node radius is ignored,
+ *      as for the PD floor.  PBD: a node with phi_k(x) < radius is pushed to phi_k = radius every iteration, and the
+ *      floor's friction rule acts on the tangential velocity.
+ *      Collider contacts are not counted in PiesB200Stats (the projection counters keep the reference's definition),
+ *      and nothing about them is read back during a tick. ---- */
+#define PIES_B200_COLLIDER_HALFSPACE 0
+#define PIES_B200_COLLIDER_SPHERE 1
+#define PIES_B200_COLLIDER_BOX 2
+#define PIES_B200_MAX_COLLIDERS 32 /* the width of the per-node contact mask */
+typedef struct PiesB200Collider { /* 64 bytes */
+  uint32_t kind;                  /* PIES_B200_COLLIDER_* */
+  float center[3];                /* half-space: a point on its plane; sphere, box: the centre */
+  float axes[9];                  /* half-space: axes[0..2] = outward normal; box: three orthonormal axes, column after column */
+  float extent[3];                /* sphere: radius in extent[0]; box: half extents */
+} PiesB200Collider;
+/* Replaces the solver's colliders (n = 0 removes all) between ticks.  EINVAL: unknown kind, non-finite value, zero normal,
+ * radius or half extent <= 0, box axes not orthonormal within 1e-4, or a call inside pd_tick_begin .. pd_tick_end;
+ * ERANGE: n > PIES_B200_MAX_COLLIDERS.  A rejected set leaves the previous one in place.  pies_b200_clear removes them. */
+int pies_b200_set_colliders(PiesB200Solver* s, uint32_t n, const PiesB200Collider* c);
+/* vertex_count() masks of the last PD detection (tick or pies_b200_detect): bit k = node in contact with collider k.
+ * All zero when the solver had no colliders then. */
+int pies_b200_get_collider_contacts(PiesB200Solver* s, uint32_t* masks);
+/* The device functions of phi and n on caller data (validated like set_colliders): for point p and collider k,
+ * phi[p * nColliders + k] and normals[3 * (p * nColliders + k) + 0..2]. */
+int pies_b200_probe_colliders(uint32_t nPoints, const float* xyz, uint32_t nColliders, const PiesB200Collider* c,
+                              float* phi, float* normals);
+
 /* ---- readback (Solver::getVertices/getLines/getTriangles; Solver.h:65-69) ---- */
 uint32_t pies_b200_vertex_count(const PiesB200Solver* s);
 uint32_t pies_b200_line_index_count(const PiesB200Solver* s);

@@ -181,6 +181,7 @@ int pies_b200_clear(PiesB200Solver* s) {
     s->builtVersion = ~0ull;
     s->stats.triCollisions = s->stats.staticCollisions = 0;
     s->stats.collisionProjections = 0;
+    s->colliderSet.clear(); s->colMaskColliders = 0;
     s->renderStateDirty = true;
     return PIES_B200_OK;
   });
@@ -418,6 +419,19 @@ int pies_b200_detect(PiesB200Solver* s) {
     rc = pies::runDetection(s, lists);
     if (rc) return rc;
     cudaStreamSynchronize(s->stream);
+    return PIES_B200_OK;
+  });
+}
+int pies_b200_set_colliders(PiesB200Solver* s, uint32_t n, const PiesB200Collider* c) {
+  return guarded(s, [&]() { return pies::setColliders(s, n, c); });
+}
+int pies_b200_get_collider_contacts(PiesB200Solver* s, uint32_t* masks) {
+  if (!s || !masks) return PIES_B200_EINVAL;
+  return guarded(s, [&]() {
+    const uint32_t n = s->scene.nodeCount();
+    if (!s->colMaskColliders || s->n != n) { std::memset(masks, 0, (size_t)n * sizeof(uint32_t)); return PIES_B200_OK; }
+    PIES_CHECK(s, cudaMemcpyAsync(masks, s->colMask.p, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+    PIES_CHECK(s, cudaStreamSynchronize(s->stream));
     return PIES_B200_OK;
   });
 }

@@ -52,7 +52,9 @@ int launchContactProject(cudaStream_t s, const ContactLists& c, const float4* q,
 // The whole right-hand side in one pass when there are contacts: the constraint gather of k_gather_rhs (pd_kernels.cu),
 // then rhs_i += sum of the collision contributions (list order) + per floor duplicate w * projectedPosition
 // (Solver.cpp:337-349), in that order; the floor contacts' projectedPosition (the position with y < 0 -> 0) is written to
-// `snap` for the stabilisation sweeps.  nodes: the nodes to assemble (null = 0 .. n-1).
+// `snap` for the stabilisation sweeps, then the static colliders' terms when kColliders.  nodes: the nodes to assemble
+// (null = 0 .. n-1).
+template <bool kColliders>
 __global__ void __launch_bounds__(kThreads) k_gather_rhs_contacts(uint32_t n, const uint32_t* __restrict__ nodes,
                                                                   const float4* __restrict__ msn,
                                                                   const int* __restrict__ incPtr,
@@ -81,7 +83,7 @@ __global__ void __launch_bounds__(kThreads) k_gather_rhs_contacts(uint32_t n, co
       acc.x += cv.x; acc.y += cv.y; acc.z += cv.z;
     }
   }
-  addContactTerms(acc, i, c, contribC, q, snap);
+  addContactTerms<kColliders>(acc, i, c, contribC, q, snap);
   acc.w = 0.0f;
   rhs[i] = acc;
 }
@@ -90,7 +92,10 @@ int launchGatherRhsContacts(cudaStream_t s, uint32_t n, const uint32_t* nodes, c
                             const uint32_t* inc, const float4* contrib, const ContactLists& c, const float4* contribC,
                             const float4* q, float4* snap, float4* rhs) {
   if (!n) return 0;
-  k_gather_rhs_contacts<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, nodes, msn, incPtr, inc, contrib, c, contribC, q, snap, rhs);
+  if (c.nCollide)
+    k_gather_rhs_contacts<true><<<gridFor(n, kThreads), kThreads, 0, s>>>(n, nodes, msn, incPtr, inc, contrib, c, contribC, q, snap, rhs);
+  else
+    k_gather_rhs_contacts<false><<<gridFor(n, kThreads), kThreads, 0, s>>>(n, nodes, msn, incPtr, inc, contrib, c, contribC, q, snap, rhs);
   return 1;
 }
 
@@ -621,7 +626,8 @@ void preloadContactKernels() {
   cudaFuncGetAttributes(&a, k_gs_mid<true>);
   cudaFuncGetAttributes(&a, k_gs_mid<false>);
   cudaFuncGetAttributes(&a, k_floor_snap);
-  cudaFuncGetAttributes(&a, k_gather_rhs_contacts);
+  cudaFuncGetAttributes(&a, k_gather_rhs_contacts<false>);
+  cudaFuncGetAttributes(&a, k_gather_rhs_contacts<true>);
   cudaFuncGetAttributes(&a, k_floor_friction);
 }
 

@@ -585,7 +585,24 @@ int detectTriangles(DetectWork& w, cudaStream_t s, const DetectInput& in, Contac
   DCHECK(w.floorW.reserve(n + 1));
   DCHECK(w.nodeDone.reserve(n + 1));
   out.floorW = w.floorW.p; out.floorMult = w.floorMult.p; out.nodeDone = w.nodeDone.p;
-  if (!nTri) return 0;
+  const uint32_t nCol = in.colliders.n;
+  // static colliders: every node's mask, their weights after the floor's (floorW), published with the lists
+  auto colliderPass = [&](bool haveFloor) {
+    if (!nCol) return;
+    L += launchColliderDetect(s, n, in.colliders, in.q, in.thickness, haveFloor, in.colMask, w.floorW.p);
+    out.nCollide = nCol; out.colMask = in.colMask;
+  };
+  if (!nTri) {
+    if (nCol && n) {  // no triangles (bare nodes, ropes): only the colliders' diagonal
+      colliderPass(false);
+      DCHECK(w.cDiag.reserve(n + 1));
+      k_ccsr_fill<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, nullptr, nullptr, nullptr, nullptr, nullptr, w.floorW.p, nullptr,
+                                                           nullptr, w.cDiag.p); ++L;
+      out.cDiag = w.cDiag.p;
+    }
+    if (launches) *launches += L;
+    return 0;
+  }
   DCHECK(w.triMin.reserve(nTri)); DCHECK(w.triRec.reserve(nTri)); DCHECK(w.cnt.reserve(nTri + 2));
   DCHECK(w.cntRank.reserve(nTri + 2)); DCHECK(w.floorRank.reserve(nTri + 2));
   DCHECK(w.aabbLo.reserve(nTri)); DCHECK(w.aabbHi.reserve(nTri));
@@ -737,7 +754,8 @@ int detectTriangles(DetectWork& w, cudaStream_t s, const DetectInput& in, Contac
     k_floor_weight<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, w.floorMult.p, w.floorW.p); ++L;
     w.floorDirty = nFloor != 0;
   }
-  if (nHit || nFloor) {
+  colliderPass(nFloor != 0);
+  if (nHit || nFloor || nCol) {
     DCHECK(w.cDiag.reserve(n + 1));
     const uint32_t nU = nHit;  // bound: the number of distinct contacts is still on its way to the host
     if (nU) {
@@ -746,7 +764,7 @@ int detectTriangles(DetectWork& w, cudaStream_t s, const DetectInput& in, Contac
       L += launchExclusiveScan(s, w.cPtr.p, n + 1, w.scanScratch.p);
     }
     k_ccsr_fill<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, nU ? w.uIncPtr.p : nullptr, w.uInc.p, w.uTri.p, w.uW.p, w.cPtr.p,
-                                                         nFloor ? w.floorW.p : nullptr, w.cCol.p, w.cVal.p, w.cDiag.p); ++L;
+                                                         (nFloor || nCol) ? w.floorW.p : nullptr, w.cCol.p, w.cVal.p, w.cDiag.p); ++L;
     out.cDiag = w.cDiag.p;
     if (nU) { out.cPtr = (int*)w.cPtr.p; out.cCol = w.cCol.p; out.cVal = w.cVal.p; }
   }

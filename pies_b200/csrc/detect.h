@@ -15,6 +15,9 @@ struct DetectInput {
   float threshold;       // collisionThresholdDistance
   float floorLimit;      // floorHeight + collisionThickness
   const uint32_t* order = nullptr;  // optional canonical-order override (device), see canonicalRank
+  ColliderSet colliders{};          // static colliders (colliders.cu): masks into colMask, weights into floorW
+  float thickness = 0.0f;           // collisionThickness
+  uint32_t* colMask = nullptr;
 };
 
 struct DetectWork {

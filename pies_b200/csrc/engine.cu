@@ -218,7 +218,7 @@ int ensureBuilt(PiesB200Solver* s) {
   if (!s->islands) s->islands = new IslandWork();
   if (uploadIslandStatics(*s->islands, st, y) != 0) return failCuda(s, s->islands->lastError, "uploadIslandStatics", __LINE__);
   preloadDetectKernels(); preloadContactKernels(); preloadReblockKernels(); preloadSortKernels(); preloadPcgKernels();
-  preloadIslandKernels();
+  preloadIslandKernels(); preloadColliderKernels();
   {
     // The per-substep collision buffers (detect.cu, reblock.cu, contact.cu) first appear, and later grow, in the middle
     // of a run; growing the stream-ordered pool there costs tens of milliseconds in one tick.  Reserve the pool once
@@ -342,6 +342,12 @@ int runDetection(PiesB200Solver* s, ContactLists& lists) {
   DetectInput in{s->triIds.p, s->q.p, s->prev.p, s->scene.triCount(), s->n, s->opt.threadCount,
                  s->opt.collisionThresholdDistance, s->opt.floorHeight + s->opt.collisionThickness,
                  (s->haveTriOrder && s->triOrder.cap >= s->scene.triCount()) ? s->triOrder.p : nullptr};
+  in.colliders = colliderSet(s);
+  in.thickness = s->opt.collisionThickness;
+  if (in.colliders.n) {
+    PIES_CHECK(s, s->colMask.reserve(s->n + 1)); PIES_CHECK(s, s->colRhs.reserve(s->n + 1));
+    in.colMask = s->colMask.p;
+  }
   int L = 0;
   lists = ContactLists{};
   if (detectTriangles(*s->detect, s->stream, in, lists, &L) != 0)
@@ -353,6 +359,8 @@ int runDetection(PiesB200Solver* s, ContactLists& lists) {
   if (prepareContactSweeps(*s->contact, s->stream, lists) < 0)
     return failCuda(s, cudaErrorMemoryAllocation, "prepareContactSweeps", __LINE__);
   if (lists.nUnique) PIES_CHECK(s, s->contact->contribC.reserve(4ull * lists.nUnique));
+  lists.colRhs = lists.nCollide ? s->colRhs.p : nullptr;
+  s->colMaskColliders = lists.nCollide;
   s->stats.triCollisions = lists.nTri;
   s->stats.staticCollisions = lists.nFloor;
   return PIES_B200_OK;
@@ -516,7 +524,7 @@ int pdIteration(PiesB200Solver* s) {
   const ContactLists& lists = c->lists;
   PdViews v = pdViews(s);
   float4* contribC = s->contact ? s->contact->contribC.p : nullptr;
-  const bool anyContact = lists.nTri || lists.nFloor;
+  const bool anyContact = lists.nTri || lists.nodeWeights();
   // The fused local step + RHS (k_tet_rhs) covers the closed segments; the elements and nodes outside them take the
   // two-kernel path.  A/B switch: PIES_B200_NO_FUSED_LOCAL sends everything through the two-kernel path.
   static const bool noFused = std::getenv("PIES_B200_NO_FUSED_LOCAL") != nullptr;
@@ -529,6 +537,8 @@ int pdIteration(PiesB200Solver* s) {
   // the local span holds the tet span (msLocal is the whole local step + RHS)
   const int spLocal = timer.begin(kPhLocal);
   s->launches += launchContactProject(st, lists, s->q.p, s->opt.collisionThickness, contribC);  // k_tet_rhs reads contribC
+  if (lists.nCollide)   // ... and colRhs
+    s->launches += launchColliderProject(st, n, colliderSet(s), lists.colMask, s->q.p, s->colRhs.p);
   // the tet slot times the tet projections of both paths, with the RHS of the segments when fused
   const int spTet = timer.begin(kPhTetKernel);
   s->launches += launchTetRhs(st, v.te, sg, s->q.p, s->msn.p, s->incPtr.p, lists, contribC, s->snap.p, s->rhs.p);
@@ -642,6 +652,7 @@ int pdSubstepEnd(PiesB200Solver* s) {
   if (s->contact)
     s->launches += launchStabilize(st, *s->contact, lists, n, s->q.p, s->prev.p, s->snap.p, o.collisionThickness,
                                    o.collisionStabilizationIterations);
+  if (lists.nCollide) s->launches += launchColliderSnap(st, n, colliderSet(s), lists.colMask, s->q.p);
   timer.end();
   s->stats.reserved = 0;
   if (s->blocks && s->blocks->countsReady && lists.nTri) {
@@ -653,6 +664,8 @@ int pdSubstepEnd(PiesB200Solver* s) {
   timer.end();
   timer.begin(kPhContact);
   if (s->contact) s->launches += launchFriction(st, *s->contact, lists, n, s->q.p, s->vel.p, o.friction, o.staticFrictionThreshold);
+  if (lists.nCollide)
+    s->launches += launchColliderFriction(st, n, colliderSet(s), lists.colMask, s->q.p, s->vel.p, o.friction, o.staticFrictionThreshold);
   timer.end();
   s->stats.collisionProjections = lists.nTri + lists.nFloor;
   ++s->stats.substepsLastTick;

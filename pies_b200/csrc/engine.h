@@ -108,6 +108,12 @@ struct PiesB200Solver {
   pies::DevBuf<uint32_t> triOrder; bool haveTriOrder = false;  // canonical-order override (slab-partitioned hosts)
   pies::DevBuf<uint32_t> ownedCount;  // output of countOwnedContacts (its own buffer: `flag` belongs to the CG reductions)
   pies::DevBuf<uint8_t> ownedMask; bool haveOwnedMask = false; // nodes this rank owns (others are ghosts)
+  // static colliders (colliders.cu): the validated set, its device copy, the per-node contact masks of the last detection
+  // (valid for colMaskColliders colliders; 0 = none) and the per-iteration sum of their weighted projections
+  std::vector<PiesB200Collider> colliderSet;
+  pies::DevBuf<PiesB200Collider> colliders;
+  pies::DevBuf<uint32_t> colMask; pies::DevBuf<float4> colRhs;
+  uint32_t colMaskColliders = 0;
 
   float* hostPacked = nullptr;  // pinned, 3 floats per node
   size_t hostPackedCap = 0;
@@ -143,6 +149,11 @@ void unregisterVertexMirror(PiesB200Solver* s);  // before anything that may rea
 int uploadStateArrays(PiesB200Solver* s, const float* pos, const float* prev, const float* vel);
 int runDetection(PiesB200Solver* s, ContactLists& lists);
 int pbdHashOnly(PiesB200Solver* s);
+// Checks a caller's collider set (include/pies_b200.h: set_colliders) into out, half-space normals normalised; on failure
+// returns PIES_B200_EINVAL / ERANGE with the reason in *why.
+int prepareColliders(uint32_t n, const PiesB200Collider* in, std::vector<PiesB200Collider>& out, const char** why);
+int setColliders(PiesB200Solver* s, uint32_t n, const PiesB200Collider* c);
+inline ColliderSet colliderSet(const PiesB200Solver* s) { return ColliderSet{s->colliders.p, (uint32_t)s->colliderSet.size()}; }
 int pbdOccupancyCounts(PiesB200Solver* s, uint64_t* nCells, uint64_t* nMembers);
 int pbdOccupancy(PiesB200Solver* s, int64_t* cellsXYZ, uint32_t* counts, uint32_t* members);
 }  // namespace pies

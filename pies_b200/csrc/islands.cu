@@ -1173,7 +1173,7 @@ int buildIslands(IslandWork& w, cudaStream_t s, uint32_t n, const CsrMatrix& S, 
     IslandArgs a{};
     a.counts = w.counts.p; a.tierDesc = w.tierDesc.p; a.listStride = w.nBodies;
     a.order = w.order.p; a.pos = w.pos.p; a.rowPtr = S.rowPtr; a.val = S.val; a.colRank = w.colRank.p; a.rankInBody = w.rankInBody.p;
-    a.cPtr = c.nUnique ? c.cPtr : nullptr; a.cCol = c.cCol; a.cVal = c.cVal; a.cDiag = (c.nTri || c.nFloor) ? c.cDiag : nullptr;
+    a.cPtr = c.nUnique ? c.cPtr : nullptr; a.cCol = c.cCol; a.cVal = c.cVal; a.cDiag = (c.nTri || c.nodeWeights()) ? c.cDiag : nullptr;
     if (w.tierCount[kDenseSlot]) ICHECK(w.denseInv.reserve((size_t)w.tierCount[kDenseSlot] * kDenseMax * kDenseMax));
     if (w.tierCount[kDenseSlot2]) ICHECK(w.denseInv2.reserve((size_t)w.tierCount[kDenseSlot2] * kDenseMax2 * kDenseMax2));
     // On the solver's stream: run beside the first local step on a side stream (r02x) they only moved their time from one
@@ -1201,7 +1201,7 @@ int launchIslandSolve(IslandWork& w, cudaStream_t s, const CsrMatrix& S, const C
   a.counts = w.counts.p; a.tierList = w.tierList.p; a.tierDesc = w.tierDesc.p; a.listStride = w.nBodies;
   a.islStart = w.islStart.p; a.order = w.order.p; a.pos = w.pos.p; a.nnzOff = w.nnzOff.p;
   a.rowPtr = S.rowPtr; a.col = S.col; a.val = S.val; a.colRank = w.colRank.p; a.rankInBody = w.rankInBody.p;
-  a.cPtr = c.nUnique ? c.cPtr : nullptr; a.cCol = c.cCol; a.cVal = c.cVal; a.cDiag = (c.nTri || c.nFloor) ? c.cDiag : nullptr;
+  a.cPtr = c.nUnique ? c.cPtr : nullptr; a.cCol = c.cCol; a.cVal = c.cVal; a.cDiag = (c.nTri || c.nodeWeights()) ? c.cDiag : nullptr;
   a.slotOf = slotOf; a.blockNodes = pw.blockNodes; a.blockInv = pw.blockInv; a.blockMeta = pw.blockMeta;
   a.blkLocal = w.blkLocal.p; a.matCol = w.matCol.p; a.matVal = w.matVal.p; a.deltaScratch = pw.delta;
   a.apScratch = pw.ap; a.zScratch = pw.z; a.slotIsl = w.slotIsl.p;

@@ -6,6 +6,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/pies_b200.h"
+
 namespace pies {
 
 // ---------------------------------------------------------------- layouts ----
@@ -69,14 +71,21 @@ struct ContactLists {
   float* floorW = nullptr;     // per node: sum of floor-contact weights (multiplicity * 1e4)
   // The same collision matrix C_t in streamable form (what the CG mat-vec reads): off-diagonal entries as CSR
   // (a point row holds -w for its three triangle corners, a corner row -w for the point; entries in incidence
-  // order) and the per-node diagonal sum (3 w / w per contact + the floor weight).  cDiag is valid when
-  // nTri || nFloor, the CSR when nUnique.
+  // order) and the per-node diagonal sum (3 w / w per contact + the floor and collider weights).  cDiag is valid
+  // when nTri || nodeWeights(), the CSR when nUnique.
   int* cPtr = nullptr; int* cCol = nullptr; float* cVal = nullptr; float* cDiag = nullptr;
   uint32_t* floorMult = nullptr;
   // ordered Gauss-Seidel sweeps: ticket[e] = position of entry e in each of its four nodes' incidence
   // lists; nodeDone[v] = entries touching v already executed in the current sweep
   uint4* ticket = nullptr;
   uint32_t* nodeDone = nullptr;
+  // Static colliders (colliders.cu): the solver's collider count when this detection wrote colMask, else 0.  A host count,
+  // not a contact count, so nothing is read back.  When it is set, floorW and cDiag also hold 1e4 per mask bit.
+  uint32_t nCollide = 0;
+  const uint32_t* colMask = nullptr;   // per node: bit k = in contact with collider k
+  const float4* colRhs = nullptr;      // per node with a mask: sum over its bits (ascending) of 1e4 p_k, this PD iteration
+  // floorW / cDiag carry one-node contact weights (floor or collider)
+  __host__ __device__ bool nodeWeights() const { return nFloor || nCollide; }
 };
 
 // ------------------------------------------------------------- PD kernels ----
@@ -97,6 +106,26 @@ int launchTetRhs(cudaStream_t s, const TetElems& e, const TetSegments& sg, const
                  const int* incPtr, const ContactLists& c, const float4* contribC, float4* snap, float4* rhs);
 int launchVelocityUpdate(cudaStream_t s, uint32_t n, const float4* q, float4* prev, float4* vel, float h,
                          float damping, float gravity);
+
+// ------------------------------------------------------ static colliders -----
+// (colliders.cu; col = the solver's device copy of its colliders, n of them)
+struct ColliderSet { const PiesB200Collider* col = nullptr; uint32_t n = 0; };
+// Detection: mask of every node (phi_k(q) < thickness), and floorW[i] = (haveFloor ? floorW[i] : 0) + 1e4 per mask bit.
+int launchColliderDetect(cudaStream_t s, uint32_t n, const ColliderSet& c, const float4* q, float thickness,
+                         bool haveFloor, uint32_t* mask, float* floorW);
+// Local step: colRhs[i] = sum over the mask bits of node i (ascending) of 1e4 p_k(q_i).
+int launchColliderProject(cudaStream_t s, uint32_t n, const ColliderSet& c, const uint32_t* mask, const float4* q,
+                          float4* colRhs);
+// After stabilisation: q of every node with a mask projected through its colliders in sequence.
+int launchColliderSnap(cudaStream_t s, uint32_t n, const ColliderSet& c, const uint32_t* mask, float4* q);
+// After the floor friction: the friction rule of k_floor_friction in each contact's tangent plane.
+int launchColliderFriction(cudaStream_t s, uint32_t n, const ColliderSet& c, const uint32_t* mask, const float4* q,
+                           float4* vel, float friction, float staticThreshold);
+// PBD: after the floor clamp / after the velocity update (radius = prev.w).
+int launchPbdColliderClamp(cudaStream_t s, uint32_t n, const ColliderSet& c, float4* q, const float4* prev);
+int launchPbdColliderFriction(cudaStream_t s, uint32_t n, const ColliderSet& c, const float4* q, const float4* prev,
+                              float4* vel, float friction);
+void preloadColliderKernels();
 
 // ------------------------------------------------------------------ PCG -----
 struct PcgWork {

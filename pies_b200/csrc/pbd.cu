@@ -872,10 +872,12 @@ int tickPBD(PiesB200Solver* s, bool refreshMirror) {
       if ((rc = sweep(s, w, w.nBend, bend))) goto done;
       if ((rc = collideNodes(s, w))) goto done;
       k_pbd_floor<<<gridFor(n, kThreads), kThreads, 0, st>>>(n, s->q.p, s->prev.p, o.floorHeight); ++s->launches;
+      s->launches += launchPbdColliderClamp(st, n, colliderSet(s), s->q.p, s->prev.p);
       s->stats.projectionsLastTick += (s->releaseHinge ? 0u : w.nPos) + w.nDist + w.nBend;
     }
     k_pbd_velocity<<<gridFor(n, kThreads), kThreads, 0, st>>>(n, s->q.p, s->prev.p, s->vel.p, dt, o.damping, o.friction,
                                                              o.floorHeight); ++s->launches;
+    s->launches += launchPbdColliderFriction(st, n, colliderSet(s), s->q.p, s->prev.p, s->vel.p, o.friction);
     ++s->stats.substepsLastTick;
   }
   s->stats.projectionsLastTick += w.visitsLastTick;

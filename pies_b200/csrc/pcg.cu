@@ -82,7 +82,7 @@ __device__ __forceinline__ void applyRowD(uint32_t i, const CsrMatrix& A, const 
     float4 xv = __ldg(x + __ldg(A.col + k));
     y[0] += a * (double)xv.x; y[1] += a * (double)xv.y; y[2] += a * (double)xv.z;
   }
-  if (c.nFloor) {
+  if (c.nodeWeights()) {
     double fw = (double)c.floorW[i];
     y[0] += fw * (double)xi.x; y[1] += fw * (double)xi.y; y[2] += fw * (double)xi.z;
   }

@@ -115,6 +115,8 @@ int launchTetElems(cudaStream_t s, const TetElems& e, const uint32_t* list, uint
 // two-kernel path, so the same bits, without the contributions' round trip through HBM and the inc gather.
 // Eight CTAs per SM (32 warps, 64 registers: a 52 B spill of loop state to L1) measured 75.0 us per iteration at S3 on a
 // B200, seven (72 registers) 77.3 us, six (78, no spill) 81.3 us; one 256-thread CTA per segment 93.6 us.
+// kColliders adds the static colliders' terms; the variant without them is launched whenever the solver has none.
+template <bool kColliders>
 __global__ void __launch_bounds__(kTetRhsThreads, 8) k_tet_rhs(TetElems e, TetSegments sg, const float4* __restrict__ q,
                                                             const float4* __restrict__ msn, const int* __restrict__ incPtr,
                                                             ContactLists c, const float4* __restrict__ contribC,
@@ -139,7 +141,7 @@ __global__ void __launch_bounds__(kTetRhsThreads, 8) k_tet_rhs(TetElems e, TetSe
       const float4 cv = sC[sg.slot[k]];
       acc.x += cv.x; acc.y += cv.y; acc.z += cv.z;
     }
-    addContactTerms(acc, i, c, contribC, q, snap);
+    addContactTerms<kColliders>(acc, i, c, contribC, q, snap);
     acc.w = 0.0f;
     rhs[i] = acc;
   }
@@ -148,7 +150,8 @@ __global__ void __launch_bounds__(kTetRhsThreads, 8) k_tet_rhs(TetElems e, TetSe
 int launchTetRhs(cudaStream_t s, const TetElems& e, const TetSegments& sg, const float4* q, const float4* msn,
                  const int* incPtr, const ContactLists& c, const float4* contribC, float4* snap, float4* rhs) {
   if (!sg.n) return 0;
-  k_tet_rhs<<<sg.n, kTetRhsThreads, 0, s>>>(e, sg, q, msn, incPtr, c, contribC, snap, rhs);
+  if (c.nCollide) k_tet_rhs<true><<<sg.n, kTetRhsThreads, 0, s>>>(e, sg, q, msn, incPtr, c, contribC, snap, rhs);
+  else k_tet_rhs<false><<<sg.n, kTetRhsThreads, 0, s>>>(e, sg, q, msn, incPtr, c, contribC, snap, rhs);
   return 1;
 }
 

@@ -223,7 +223,7 @@ __global__ void __launch_bounds__(kFactorWarps * 32) k_block_factor(uint32_t nSt
       if ((sj >> 5) == b) row[sj & 31u] = S.val[k];
     }
     float diag = row[lane];
-    if (c.nFloor) diag += c.floorW[node];
+    if (c.nodeWeights()) diag += c.floorW[node];
     if (c.nUnique) {
       for (int k = c.incPtr[node]; k < c.incPtr[node + 1]; ++k) {
         uint32_t v = c.inc[k];
@@ -349,7 +349,7 @@ int rebuildBlocks(BlockWork& w, cudaStream_t s, uint32_t n, const CsrMatrix& S, 
     RCHECK(w.scanScratch.reserve(scanScratchElems(std::max<uint64_t>(n + 2, w.scanCap))));
   }
   k_static_membership<<<gridFor((uint64_t)nStatic * 32, kThreads), kThreads, 0, s>>>(nStatic, staticNodes, w.flag.p, c.floorW,
-                                                                                    c.nFloor ? 1 : 0, w.blockNodes.p,
+                                                                                    c.nodeWeights() ? 1 : 0, w.blockNodes.p,
                                                                                     w.slotOf.p, w.blockCount.p, w.dirty.p); ++L;
   k_assign_dynamic<<<gridFor(std::max(nT, 1u), kThreads), kThreads, 0, s>>>(nT, nStatic, w.heads.p + nT, w.heads.p, w.start.p,
                                                                            w.blkOff.p, w.vals.p, w.blockNodes.p, w.slotOf.p,

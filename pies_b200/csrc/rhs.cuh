@@ -12,7 +12,9 @@ constexpr float kFloorW = 10000.0f;  // StaticCollisionConstraint::w (CollisionC
 
 // acc += the collision contributions of node i (list order), then w * projectedPosition once per floor duplicate; the
 // floor contacts' projectedPosition (the position with y < 0 -> 0) is written to `snap` for the stabilisation sweeps.
+// kColliders: then the static colliders' terms, c.colRhs[i] (formed by k_collider_project), for a node with a mask.
 // A no-op when the substep has no contacts.
+template <bool kColliders>
 __device__ __forceinline__ void addContactTerms(float4& acc, uint32_t i, const ContactLists& c,
                                                 const float4* __restrict__ contribC, const float4* __restrict__ q,
                                                 float4* __restrict__ snap) {
@@ -28,6 +30,10 @@ __device__ __forceinline__ void addContactTerms(float4& acc, uint32_t i, const C
     if (p.y < 0.0f) p.y = 0.0f;
     snap[i] = p;
     for (uint32_t k = 0; k < mult; ++k) { acc.x += kFloorW * p.x; acc.y += kFloorW * p.y; acc.z += kFloorW * p.z; }
+  }
+  if (kColliders && c.colMask[i]) {
+    const float4 p = c.colRhs[i];
+    acc.x += p.x; acc.y += p.y; acc.z += p.z;
   }
 }
 

@@ -59,6 +59,51 @@ class Stats(C.Structure):
     ]
 
 
+COLLIDER_HALFSPACE, COLLIDER_SPHERE, COLLIDER_BOX = 0, 1, 2
+MAX_COLLIDERS = 32  # the width of the per-node contact mask
+
+
+class Collider(C.Structure):
+    """PiesB200Collider (include/pies_b200.h), 64 bytes: a static half-space, sphere or oriented solid box."""
+    _fields_ = [("kind", C.c_uint32), ("center", C.c_float * 3), ("axes", C.c_float * 9), ("extent", C.c_float * 3)]
+
+
+def halfspace(point, normal):
+    """The half-space below the plane through `point` with outward `normal` (normalised here and again by the library)."""
+    n = np.asarray(normal, np.float64).reshape(3)
+    length = float(np.linalg.norm(n))
+    if length > 0.0:
+        n = n / length
+    c = Collider(kind=COLLIDER_HALFSPACE)
+    c.center[:] = [float(x) for x in np.asarray(point, np.float64).reshape(3)]
+    c.axes[:] = [float(x) for x in n] + [0.0] * 6
+    return c
+
+
+def sphere(center, radius):
+    c = Collider(kind=COLLIDER_SPHERE)
+    c.center[:] = [float(x) for x in np.asarray(center, np.float64).reshape(3)]
+    c.extent[:] = [float(radius), 0.0, 0.0]
+    return c
+
+
+def box(center, half_extents, axes=None):
+    """Solid box; axes: 3 x 3 whose COLUMNS are the box's orthonormal local axes (default: the world axes)."""
+    a = np.eye(3) if axes is None else np.asarray(axes, np.float64).reshape(3, 3)
+    c = Collider(kind=COLLIDER_BOX)
+    c.center[:] = [float(x) for x in np.asarray(center, np.float64).reshape(3)]
+    c.axes[:] = [float(x) for x in a.T.reshape(9)]   # column after column
+    c.extent[:] = [float(x) for x in np.asarray(half_extents, np.float64).reshape(3)]
+    return c
+
+
+def _collider_array(colliders):
+    arr = (Collider * max(1, len(colliders)))()
+    for i, c in enumerate(colliders):
+        arr[i] = c
+    return arr
+
+
 VERTEX_DTYPE = np.dtype([("position", np.float32, 3), ("radius", np.float32),
                          ("baseColor", np.float32, 3), ("roughness", np.float32),
                          ("metallic", np.float32)])  # Solver::Vertex, 36 bytes
@@ -149,6 +194,9 @@ _SIGNATURES = {
     "pies_b200_probe_node_range": (C.c_int, [C.c_uint32, _f32p, _f32p, C.c_float, _i64p, _u32p]),
     "pies_b200_probe_sort_pairs": (C.c_int, [C.c_uint64, _u64p, _u32p, C.c_int]),
     "pies_b200_probe_sell": (C.c_int, [C.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(C.c_uint64)]),
+    "pies_b200_set_colliders": (C.c_int, [_vp, C.c_uint32, _vp]),
+    "pies_b200_get_collider_contacts": (C.c_int, [_vp, _u32p]),
+    "pies_b200_probe_colliders": (C.c_int, [C.c_uint32, _vp, C.c_uint32, _vp, _vp, _vp]),
     "pies_b200_probe_segments": (C.c_int, [C.c_uint32, _vp, C.c_uint32, _vp, C.c_uint32, _vp, _u64p] + [_vp] * 7),
 }
 
@@ -433,6 +481,18 @@ class Solver:
             self._ck(lib().pies_b200_debug_island_trace(self.h, int(slot), out.ctypes.data_as(C.c_void_p), cnt.value, C.byref(cnt)))
         return out
 
+    def setColliders(self, colliders):
+        """Replaces the static colliders (a list of Collider, e.g. from halfspace / sphere / box; [] removes all)."""
+        colliders = list(colliders)
+        self._ck(lib().pies_b200_set_colliders(self.h, len(colliders), C.cast(_collider_array(colliders), _vp)))
+
+    def colliderContacts(self):
+        """Per node, the collider contact mask of the last PD detection (bit k = in contact with collider k)."""
+        out = np.zeros(lib().pies_b200_vertex_count(self.h), np.uint32)
+        if len(out):
+            self._ck(lib().pies_b200_get_collider_contacts(self.h, out))
+        return out
+
     def staticCollisions(self):
         out = np.empty(lib().pies_b200_static_collision_count(self.h), dtype=np.uint32)
         self._ck(lib().pies_b200_get_static_collisions(self.h, out))
@@ -613,6 +673,19 @@ def probe_sell(rowPtr, col, val):
     sc = np.zeros(padded.value, np.int32); sv = np.zeros(padded.value, np.float32)
     _ckp(lib().pies_b200_probe_sell(n, p(rp), p(c), p(v), p(sp), p(sr), p(sc), p(sv), C.byref(padded)))
     return sp, sr, sc, sv
+
+
+def probe_colliders(points, colliders):
+    """(phi[nPoints, nColliders], normals[nPoints, nColliders, 3]) of the library's device functions."""
+    p = np.ascontiguousarray(points, np.float32).reshape(-1, 3)
+    colliders = list(colliders)
+    phi = np.zeros((len(p), len(colliders)), np.float32)
+    nrm = np.zeros((len(p), len(colliders), 3), np.float32)
+    rc = lib().pies_b200_probe_colliders(len(p), p.ctypes.data_as(_vp), len(colliders), C.cast(_collider_array(colliders), _vp),
+                                         phi.ctypes.data_as(_vp), nrm.ctypes.data_as(_vp))
+    if rc != 0:
+        raise PiesError("pies_b200_probe_colliders failed: %d" % rc)
+    return phi, nrm
 
 
 def probe_segments(cmds, mesh_points=None, mesh_tets=None):
