@@ -195,6 +195,32 @@ int pies_b200_get_collider_contacts(PiesB200Solver* s, uint32_t* masks);
 int pies_b200_probe_colliders(uint32_t nPoints, const float* xyz, uint32_t nColliders, const PiesB200Collider* c,
                               float* phi, float* normals);
 
+/* ---- [additive] picking and dragging (DESIGN.md section 10): what an interactive host needs to click a body and pull it.
+ *
+ * Drag targets: one-node position constraints whose target and weight the host replaces between ticks, without a
+ * topology rebuild (DESIGN.md section 10).  Each call replaces the whole set (n = 0 removes it); the set persists across
+ * ticks until replaced, stays valid when bodies are appended, and pies_b200_clear removes it.  The arrays are copied
+ * before the call returns.  EINVAL: a node id >= vertex_count(), a duplicate id, a non-finite target or weight, a
+ * weight <= 0, a null array with n > 0, or a call inside pd_tick_begin .. pd_tick_end; a rejected set leaves the
+ * previous one in place.
+ *   PD: each drag is a PositionConstraint of weight w and target g for the substep: w joins the node's one-node weight
+ *       (after the floor's and the colliders') in the diagonal of the global step, and w g its right-hand side.
+ *   PBD: every iteration, right after the position-constraint sweep (also with release_hinge), x += min(w, 1) (g - x).
+ *   Drags take no part in stabilisation or friction, ignore release_hinge and are not counted in PiesB200Stats.
+ *   Without a set, every kernel computes what it computed before drags existed. */
+int pies_b200_set_drag_targets(PiesB200Solver* s, uint32_t n, const uint32_t* nodes, const float* targets /* 3n */,
+                               const float* weights /* n */);
+/* Closest hit of each ray o + t d, 0 <= t <= tMax[r], against the solver's triangles at the positions get_vertices()
+ * returns (two-sided; d need not be normalised, t is in units of d).  tri[r] = index into get_triangles() / 3 of the hit
+ * with the smallest t, ties to the lowest index, -1 on a miss; t[r] = +inf on a miss; uv[2r], uv[2r+1] = barycentric
+ * weights of corners 1 and 2 of that triangle (0 on a miss).  Moller-Trumbore in fp32 (operation order in DESIGN.md
+ * section 10); a triangle parallel to the ray or of zero area never hits.  Sees set_state without a tick, marks nothing
+ * dirty, and returns when the results are on the host.  Cost: nRays x triangle_count() ray-triangle tests (no
+ * acceleration structure).  EINVAL: a non-finite origin, a zero or non-finite direction, a NaN or negative tMax (+inf is
+ * allowed), or a null array with nRays > 0.  A scene without triangles returns all misses. */
+int pies_b200_raycast(PiesB200Solver* s, uint32_t nRays, const float* origins /* 3 per ray */, const float* dirs /* 3 per ray */,
+                      const float* tMax, int32_t* tri, float* t, float* uv /* 2 per ray */);
+
 /* ---- readback (Solver::getVertices/getLines/getTriangles; Solver.h:65-69) ---- */
 uint32_t pies_b200_vertex_count(const PiesB200Solver* s);
 uint32_t pies_b200_line_index_count(const PiesB200Solver* s);

@@ -182,6 +182,7 @@ int pies_b200_clear(PiesB200Solver* s) {
     s->stats.triCollisions = s->stats.staticCollisions = 0;
     s->stats.collisionProjections = 0;
     s->colliderSet.clear(); s->colMaskColliders = 0;
+    s->dragCount = 0;
     s->renderStateDirty = true;
     return PIES_B200_OK;
   });
@@ -434,6 +435,13 @@ int pies_b200_get_collider_contacts(PiesB200Solver* s, uint32_t* masks) {
     PIES_CHECK(s, cudaStreamSynchronize(s->stream));
     return PIES_B200_OK;
   });
+}
+int pies_b200_set_drag_targets(PiesB200Solver* s, uint32_t n, const uint32_t* nodes, const float* targets, const float* weights) {
+  return guarded(s, [&]() { return pies::setDragTargets(s, n, nodes, targets, weights); });
+}
+int pies_b200_raycast(PiesB200Solver* s, uint32_t nRays, const float* origins, const float* dirs, const float* tMax,
+                      int32_t* tri, float* t, float* uv) {
+  return guarded(s, [&]() { return pies::raycast(s, nRays, origins, dirs, tMax, tri, t, uv); });
 }
 uint32_t pies_b200_tri_collision_count(const PiesB200Solver* s) { return s ? s->stats.triCollisions : 0; }
 uint32_t pies_b200_static_collision_count(const PiesB200Solver* s) { return s ? s->stats.staticCollisions : 0; }

@@ -592,9 +592,23 @@ int detectTriangles(DetectWork& w, cudaStream_t s, const DetectInput& in, Contac
     L += launchColliderDetect(s, n, in.colliders, in.q, in.thickness, haveFloor, in.colMask, w.floorW.p);
     out.nCollide = nCol; out.colMask = in.colMask;
   };
+  const uint32_t nDrag = in.drags.n;
+  // drag targets: their weights after the floor's and the colliders' (floorW is zeroed first when neither wrote it this
+  // substep), and w g into msn, in one launch
+  auto dragPass = [&](bool haveFloorW) -> cudaError_t {
+    if (!nDrag) return cudaSuccess;
+    if (!haveFloorW) {
+      const cudaError_t e = cudaMemsetAsync(w.floorW.p, 0, (size_t)n * sizeof(float), s);
+      if (e != cudaSuccess) return e;
+    }
+    L += launchDragTerms(s, in.drags, w.floorW.p, in.msn);
+    out.nDrag = nDrag;
+    return cudaSuccess;
+  };
   if (!nTri) {
-    if (nCol && n) {  // no triangles (bare nodes, ropes): only the colliders' diagonal
+    if ((nCol || nDrag) && n) {  // no triangles (bare nodes, ropes): only the colliders' and drags' diagonal
       colliderPass(false);
+      DCHECK(dragPass(nCol != 0));
       DCHECK(w.cDiag.reserve(n + 1));
       k_ccsr_fill<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, nullptr, nullptr, nullptr, nullptr, nullptr, w.floorW.p, nullptr,
                                                            nullptr, w.cDiag.p); ++L;
@@ -755,7 +769,8 @@ int detectTriangles(DetectWork& w, cudaStream_t s, const DetectInput& in, Contac
     w.floorDirty = nFloor != 0;
   }
   colliderPass(nFloor != 0);
-  if (nHit || nFloor || nCol) {
+  DCHECK(dragPass(nFloor || nCol));
+  if (nHit || nFloor || nCol || nDrag) {
     DCHECK(w.cDiag.reserve(n + 1));
     const uint32_t nU = nHit;  // bound: the number of distinct contacts is still on its way to the host
     if (nU) {
@@ -764,7 +779,8 @@ int detectTriangles(DetectWork& w, cudaStream_t s, const DetectInput& in, Contac
       L += launchExclusiveScan(s, w.cPtr.p, n + 1, w.scanScratch.p);
     }
     k_ccsr_fill<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, nU ? w.uIncPtr.p : nullptr, w.uInc.p, w.uTri.p, w.uW.p, w.cPtr.p,
-                                                         (nFloor || nCol) ? w.floorW.p : nullptr, w.cCol.p, w.cVal.p, w.cDiag.p); ++L;
+                                                         (nFloor || nCol || nDrag) ? w.floorW.p : nullptr, w.cCol.p, w.cVal.p,
+                                                         w.cDiag.p); ++L;
     out.cDiag = w.cDiag.p;
     if (nU) { out.cPtr = (int*)w.cPtr.p; out.cCol = w.cCol.p; out.cVal = w.cVal.p; }
   }

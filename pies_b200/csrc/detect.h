@@ -18,6 +18,8 @@ struct DetectInput {
   ColliderSet colliders{};          // static colliders (colliders.cu): masks into colMask, weights into floorW
   float thickness = 0.0f;           // collisionThickness
   uint32_t* colMask = nullptr;
+  DragSet drags{};                  // drag targets (pick.cu): weights into floorW after the colliders', w g into msn
+  float4* msn = nullptr;
 };
 
 struct DetectWork {

@@ -348,6 +348,8 @@ int runDetection(PiesB200Solver* s, ContactLists& lists) {
     PIES_CHECK(s, s->colMask.reserve(s->n + 1)); PIES_CHECK(s, s->colRhs.reserve(s->n + 1));
     in.colMask = s->colMask.p;
   }
+  in.drags = dragSet(s);
+  in.msn = s->msn.p;
   int L = 0;
   lists = ContactLists{};
   if (detectTriangles(*s->detect, s->stream, in, lists, &L) != 0)

@@ -114,6 +114,11 @@ struct PiesB200Solver {
   pies::DevBuf<PiesB200Collider> colliders;
   pies::DevBuf<uint32_t> colMask; pies::DevBuf<float4> colRhs;
   uint32_t colMaskColliders = 0;
+  // drag targets (pick.cu): the validated set's size and its device copy (node ids, (g, w)); dragCount = 0 = none
+  uint32_t dragCount = 0;
+  pies::DevBuf<uint32_t> dragNode; pies::DevBuf<float4> dragTargetW;
+  // raycast staging (pick.cu): rays (2 float4 each), per-ray hit keys, packed results
+  pies::DevBuf<float4> rays; pies::DevBuf<unsigned long long> rayKey; pies::DevBuf<float4> rayHit;
 
   float* hostPacked = nullptr;  // pinned, 3 floats per node
   size_t hostPackedCap = 0;
@@ -154,6 +159,10 @@ int pbdHashOnly(PiesB200Solver* s);
 int prepareColliders(uint32_t n, const PiesB200Collider* in, std::vector<PiesB200Collider>& out, const char** why);
 int setColliders(PiesB200Solver* s, uint32_t n, const PiesB200Collider* c);
 inline ColliderSet colliderSet(const PiesB200Solver* s) { return ColliderSet{s->colliders.p, (uint32_t)s->colliderSet.size()}; }
+int setDragTargets(PiesB200Solver* s, uint32_t n, const uint32_t* nodes, const float* targets, const float* weights);
+inline DragSet dragSet(const PiesB200Solver* s) { return DragSet{s->dragNode.p, s->dragTargetW.p, s->dragCount}; }
+int raycast(PiesB200Solver* s, uint32_t nRays, const float* origins, const float* dirs, const float* tMax, int32_t* tri,
+            float* t, float* uv);
 int pbdOccupancyCounts(PiesB200Solver* s, uint64_t* nCells, uint64_t* nMembers);
 int pbdOccupancy(PiesB200Solver* s, int64_t* cellsXYZ, uint32_t* counts, uint32_t* members);
 }  // namespace pies

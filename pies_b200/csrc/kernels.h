@@ -82,10 +82,13 @@ struct ContactLists {
   // Static colliders (colliders.cu): the solver's collider count when this detection wrote colMask, else 0.  A host count,
   // not a contact count, so nothing is read back.  When it is set, floorW and cDiag also hold 1e4 per mask bit.
   uint32_t nCollide = 0;
+  // Drag targets (pick.cu): the solver's drag count when this detection added their weights to floorW and cDiag (and
+  // w g to msn), else 0.  Also a host count; it fills the padding before colMask, so the struct keeps its size.
+  uint32_t nDrag = 0;
   const uint32_t* colMask = nullptr;   // per node: bit k = in contact with collider k
   const float4* colRhs = nullptr;      // per node with a mask: sum over its bits (ascending) of 1e4 p_k, this PD iteration
-  // floorW / cDiag carry one-node contact weights (floor or collider)
-  __host__ __device__ bool nodeWeights() const { return nFloor || nCollide; }
+  // floorW / cDiag carry one-node weights (floor, collider or drag)
+  __host__ __device__ bool nodeWeights() const { return nFloor || nCollide || nDrag; }
 };
 
 // ------------------------------------------------------------- PD kernels ----
@@ -126,6 +129,14 @@ int launchPbdColliderClamp(cudaStream_t s, uint32_t n, const ColliderSet& c, flo
 int launchPbdColliderFriction(cudaStream_t s, uint32_t n, const ColliderSet& c, const float4* q, const float4* prev,
                               float4* vel, float friction);
 void preloadColliderKernels();
+
+// ---------------------------------------------------------- drag targets -----
+// (pick.cu; node[k] with targetW[k] = (g, w), ids unique)
+struct DragSet { const uint32_t* node = nullptr; const float4* targetW = nullptr; uint32_t n = 0; };
+// PD detection, after the floor and collider weights: floorW[node] += w, msn[node] += w g.
+int launchDragTerms(cudaStream_t s, const DragSet& d, float* floorW, float4* msn);
+// PBD, after the position-constraint sweep: x += min(w, 1) (g - x).
+int launchPbdDrag(cudaStream_t s, const DragSet& d, float4* q);
 
 // ------------------------------------------------------------------ PCG -----
 struct PcgWork {

@@ -868,6 +868,7 @@ int tickPBD(PiesB200Solver* s, bool refreshMirror) {
     k_pbd_advect<<<gridFor(n, kThreads), kThreads, 0, st>>>(n, s->q.p, s->prev.p, s->vel.p, dt, o.gravity); ++s->launches;
     for (uint32_t it = 0; it < o.iterations; ++it) {
       if (!s->releaseHinge && (rc = sweep(s, w, w.nPos, pos))) goto done;
+      s->launches += launchPbdDrag(st, dragSet(s), s->q.p);
       if ((rc = sweep(s, w, w.nDist, dist))) goto done;
       if ((rc = sweep(s, w, w.nBend, bend))) goto done;
       if ((rc = collideNodes(s, w))) goto done;

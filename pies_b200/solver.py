@@ -197,6 +197,8 @@ _SIGNATURES = {
     "pies_b200_set_colliders": (C.c_int, [_vp, C.c_uint32, _vp]),
     "pies_b200_get_collider_contacts": (C.c_int, [_vp, _u32p]),
     "pies_b200_probe_colliders": (C.c_int, [C.c_uint32, _vp, C.c_uint32, _vp, _vp, _vp]),
+    "pies_b200_set_drag_targets": (C.c_int, [_vp, C.c_uint32, _vp, _vp, _vp]),
+    "pies_b200_raycast": (C.c_int, [_vp, C.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "pies_b200_probe_segments": (C.c_int, [C.c_uint32, _vp, C.c_uint32, _vp, C.c_uint32, _vp, _u64p] + [_vp] * 7),
 }
 
@@ -492,6 +494,31 @@ class Solver:
         if len(out):
             self._ck(lib().pies_b200_get_collider_contacts(self.h, out))
         return out
+
+    def setDragTargets(self, nodes, targets, weights):
+        """Replaces the drag targets: node ids, their targets (n x 3) and weights (n,).  Empty arrays remove the set."""
+        ids = np.ascontiguousarray(nodes, dtype=np.uint32).reshape(-1)
+        g = np.ascontiguousarray(targets, dtype=np.float32).reshape(-1, 3)
+        w = np.ascontiguousarray(np.broadcast_to(np.asarray(weights, np.float32), ids.shape))
+        if len(g) != len(ids):
+            raise ValueError("setDragTargets: %d nodes but %d targets" % (len(ids), len(g)))
+        p = lambda a: a.ctypes.data_as(_vp) if a.size else None
+        self._ck(lib().pies_b200_set_drag_targets(self.h, len(ids), p(ids), p(g), p(w)))
+
+    def raycast(self, origins, dirs, tMax=np.inf):
+        """Closest hit of each ray o + t d (0 <= t <= tMax) against the triangles at the current positions:
+        (tri int32 (n,), -1 on a miss; t float32 (n,), +inf on a miss; uv float32 (n, 2), the barycentric weights of
+        corners 1 and 2 of the hit triangle)."""
+        o = np.ascontiguousarray(origins, dtype=np.float32).reshape(-1, 3)
+        d = np.ascontiguousarray(dirs, dtype=np.float32).reshape(-1, 3)
+        n = len(o)
+        if len(d) != n:
+            raise ValueError("raycast: %d origins but %d directions" % (n, len(d)))
+        tm = np.ascontiguousarray(np.broadcast_to(np.asarray(tMax, np.float32), (n,)))
+        tri = np.full(n, -1, np.int32); t = np.full(n, np.inf, np.float32); uv = np.zeros((n, 2), np.float32)
+        p = lambda a: a.ctypes.data_as(_vp) if a.size else None
+        self._ck(lib().pies_b200_raycast(self.h, n, p(o), p(d), p(tm), p(tri), p(t), p(uv)))
+        return tri, t, uv
 
     def staticCollisions(self):
         out = np.empty(lib().pies_b200_static_collision_count(self.h), dtype=np.uint32)
