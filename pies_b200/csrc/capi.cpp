@@ -483,12 +483,12 @@ int pies_b200_get_collision_csr(PiesB200Solver* s, uint64_t* nnz, int32_t* cPtr,
   });
 }
 int pies_b200_debug_island_trace(PiesB200Solver* s, int slot, uint32_t* out4, uint32_t cap, uint32_t* count) {
-  if (!s || !count || slot < 0 || slot >= pies::kIslandSlots) return PIES_B200_EINVAL;
+  if (!s || !count || slot < 0 || slot >= pies::kIslandLists) return PIES_B200_EINVAL;
   return guarded(s, [&]() {
     cudaSetDevice(s->device);
     *count = 0;
     if (!s->islands || !s->islands->trace.p) return fail(s, PIES_B200_EINVAL, "island trace is off: set PIES_B200_ISLAND_TRACE before the first tick");
-    const uint32_t have = s->islands->tierCount[slot];
+    const uint32_t have = s->islands->listCount[slot];
     *count = have;
     const uint32_t take = std::min(have, cap);
     if (take && out4) {

@@ -491,22 +491,14 @@ int pdSubstepBegin(PiesB200Solver* s) {
     s->launches += LC;
     // islands of S + C_t: which solves stay inside one warp / one CTA (islands.cu)
     if (s->islands) {
-      // tier 3 (one 1024-thread CTA per island of up to 7 168 nodes) is opt-in: a handful of such islands keep single SMs
-      // busy for milliseconds, the grid-wide CG spreads them over the whole device
-      const uint32_t avail = (s->tune.reserved & 256u) ? 0xFu : 0x7u;
-      const uint32_t tiers = (s->tune.reserved & 4u) ? 0u : (avail & ~((s->tune.reserved >> 4) & 0xFu));
       int LI = 0;
-      if (buildIslands(*s->islands, st, n, v.A, c->lists, bw.slotOf.p, bw.blockCount.p, bw.nBlocksBound, tiers, &LI) != 0) {
+      if (buildIslands(*s->islands, st, n, v.A, c->lists, bw.slotOf.p, bw.blockCount.p, bw.nBlocksBound, s->tune.reserved, &LI) != 0) {
         cudaError_t e = s->islands->lastError;
         pdAbort(s);
         return failCuda(s, e, "buildIslands", __LINE__);
       }
       s->launches += LI;
-      for (int t = 0; t < kIslandTiers; ++t) s->stats.islandsTier[t] = s->islands->tierCount[t];
-      s->stats.islandsTier[1] += s->islands->tierCount[kSmallCtaSlot] + s->islands->tierCount[kDenseSlot] + s->islands->tierCount[kDenseSlot2];
-      s->stats.islandsGlobal = s->islands->nLeftIslands;
-      s->stats.islandInverseFloats = s->islands->inverseFloats;
-      s->stats.islandNodesGlobal = s->islands->nLeftNodes;
+      islandStats(*s->islands, s->stats);
     }
   }
   timer.end();
@@ -572,9 +564,7 @@ int pdIteration(PiesB200Solver* s) {
   bool gridWide = true;
   if (s->islands && s->blocks) {
     IslandWork& iw = *s->islands;
-    bool any = false;
-    for (int t = 0; t < kIslandSlots; ++t) any = any || iw.tierCount[t];
-    if (any) {
+    if (iw.anyLocal()) {
       const int spIsl = timer.begin(kPhIslandKernel);
       s->launches += launchIslandSolve(iw, st, v.A, lists, v.pw, s->blocks->slotOf.p, s->rhs.p, s->q.p, s->tune.pcgTolerance,
                                        s->tune.pcgMaxIterations, solveSlot);

@@ -116,9 +116,43 @@ __global__ void __launch_bounds__(kThreads) k_isl_nodes(uint32_t n, const uint32
   nnzOff[p] = len;
 }
 
-struct IslandTierTable { IslandCaps caps[kIslandSlots]; uint32_t enabled; };
+// ------------------------------------------------------------------------------------------------- lists -----
+// An island goes to the first list of kClassifyOrder whose public tier is on and whose caps it fits, or to the grid-wide
+// CG (device list kIslandLists).  The public tier is the islandsTier entry of PiesB200Stats and the tuning bit 16 << tier.
+enum IslandKind : int { kDirect, kDense, kCtaCg, kBig };   // k_island_direct / _invert + _dense / _pcg / _pcg_big
+constexpr uint32_t kDenseMax = 128;   // node caps of the dense lists; the inverse is stored with this leading dimension
+constexpr uint32_t kDenseMax2 = 192;
+struct IslandCaps { uint32_t maxNodes, maxNnz, maxInv, maxBlocks; };
+// A/B switches that take lists out (environment, read once per process): PIES_B200_NO_SMALL_CTA, _NO_DENSE, _NO_DENSE2
+constexpr uint32_t kNoSmallCta = 1, kNoDense = 2, kNoDense2 = 4;
+struct IslandList {
+  IslandKind kind;      // also which inverse a solve reads: the packed block inverse, the dense one, the blocks' ones
+  int team, rpt;        // threads of the team solving one island, rows per thread
+  IslandCaps caps;      // nodes, matrix entries, inverse floats, blocks resident in shared memory
+  int tier;             // public tier
+  int ctasPerSm;        // grid cap of a solve
+  int shortList;        // a list that fits one wave of this list's CTAs goes to its team: a short list is latency bound
+  uint32_t offBy;       // A/B switches
+};
+constexpr IslandList kLists[kIslandLists] = {
+    {kDirect, 32, 1, {32u, 640u, 576u, 4u}, 0, 4, 0, 0u},            // 0: every free body; eight warps per CTA
+    {kCtaCg, 320, 2, {640u, 6656u, 9216u, 96u}, 1, 2, 1, 0u},
+    {kCtaCg, 512, 2, {1024u, 12288u, 17408u, 192u}, 2, 1, 2, 0u},   // 2: the whole shared memory of an SM
+    {kBig, 1024, 0, {7168u, 0u, 0u, 0u}, 3, 1, 3, 0u},               // 3: opt-in
+    // 4: the typical S3 contact island is five bodies (~140 rows), which leaves more than half of a 320-thread CTA
+    //    waiting at every barrier: 43 KB of shared memory, five CTAs per SM
+    {kCtaCg, 128, 2, {256u, 2816u, 3456u, 32u}, 1, 5, 1, kNoSmallCta},
+    {kDense, (int)kDenseMax, 1, {kDenseMax, 0u, 0u, 0u}, 1, 16, 5, kNoDense},                 // 5: 3-4 bodies of a column
+    // 6: 5-7 bodies (S3 ticks 79..100); beyond that the m^3 of the inversion and the m^2 of every apply lose to the CG
+    {kDense, (int)kDenseMax2, 1, {kDenseMax2, 0u, 0u, 0u}, 1, 10, 6, kNoDense | kNoDense2},
+};
+constexpr int kClassifyOrder[kIslandLists] = {0, 5, 6, 4, 1, 2, 3};   // cheapest solve first
+constexpr int kLaunchOrder[kIslandLists] = {3, 2, 1, 4, 6, 5, 0};     // longest chains first
 
-__global__ void __launch_bounds__(kThreads) k_isl_classify(const uint32_t* counts0, IslandTierTable tt,
+// the lists in classification order, with their numbers, as the A/B switches and the tuning word leave them
+struct IslandClassifyTable { IslandList list[kIslandLists]; int id[kIslandLists]; uint32_t tiersOn; };
+
+__global__ void __launch_bounds__(kThreads) k_isl_classify(const uint32_t* counts0, IslandClassifyTable tt,
                                                            const uint32_t* __restrict__ islStart,
                                                            const uint32_t* __restrict__ nnzOff, const uint32_t* __restrict__ order,
                                                            const uint32_t* __restrict__ slotOf,
@@ -129,25 +163,25 @@ __global__ void __launch_bounds__(kThreads) k_isl_classify(const uint32_t* count
   if (isl >= counts0[0]) return;
   const uint32_t s0 = islStart[isl], m = islStart[isl + 1] - s0;
   const uint32_t nnz = nnzOff[s0 + m] - nnzOff[s0];
-  int tier = kIslandSlots;
-  const int tryOrder[kIslandSlots] = {0, kDenseSlot, kDenseSlot2, kSmallCtaSlot, 1, 2, 3};  // cheapest solve first
+  int list = kIslandLists;
+  IslandKind kind = kCtaCg;
 #pragma unroll
-  for (int o = 0; o < kIslandSlots; ++o) {
-    const int t = tryOrder[o];
-    if (!((tt.enabled >> (t >= kSmallCtaSlot ? 1 : t)) & 1u)) continue;
-    if (m > tt.caps[t].maxNodes || (tt.caps[t].maxNnz && nnz > tt.caps[t].maxNnz)) continue;
-    if (t == 0 && blockCount[slotOf[order[s0]] >> 5] != m) continue;  // the warp tier wants the island in ONE preconditioner block
-    tier = t;
+  for (int o = 0; o < kIslandLists; ++o) {
+    const IslandList& e = tt.list[o];
+    if (!((tt.tiersOn >> e.tier) & 1u)) continue;
+    if (m > e.caps.maxNodes || (e.caps.maxNnz && nnz > e.caps.maxNnz)) continue;
+    if (e.kind == kDirect && blockCount[slotOf[order[s0]] >> 5] != m) continue;  // the island must be ONE preconditioner block
+    list = tt.id[o];
+    kind = e.kind;
     break;
   }
-  const uint32_t at = atomicAdd(counts + 1 + tier, 1u);  // list order only decides scheduling: islands are independent
-  tierList[(size_t)tier * listStride + at] = isl;
+  const uint32_t at = atomicAdd(counts + 1 + list, 1u);  // list order only decides scheduling: islands are independent
+  tierList[(size_t)list * listStride + at] = isl;
   // everything a team needs to start on the island in one 16 B record (it prefetches the next one while it solves)
-  tierDesc[(size_t)tier * listStride + at] = make_uint4(isl, s0, m, nnzOff[s0]);
-  if (tier == kIslandSlots) atomicAdd(counts + 2 + kIslandSlots, m);
-  // floats of inverse the island's solve has to read: the packed block inverse (warp list), the dense inverse (dense
-  // lists), the packed inverses of its blocks (CG lists: at most 16.5 per node, taken as 14 = a 27-node block)
-  else atomicAdd(counts + 3 + kIslandSlots, tier == 0 ? m * (m + 1u) / 2u : ((tier == kDenseSlot || tier == kDenseSlot2) ? m * m : 14u * m));
+  tierDesc[(size_t)list * listStride + at] = make_uint4(isl, s0, m, nnzOff[s0]);
+  if (list == kIslandLists) atomicAdd(counts + 2 + kIslandLists, m);
+  // floats of inverse the island's solve has to read (CG lists: at most 16.5 per node, taken as 14 = a 27-node block)
+  else atomicAdd(counts + 3 + kIslandLists, kind == kDirect ? m * (m + 1u) / 2u : (kind == kDense ? m * m : 14u * m));
 }
 
 // Marks the nodes of the islands left to the grid-wide CG, the 256-row windows that hold one and their preconditioner
@@ -156,7 +190,7 @@ __global__ void __launch_bounds__(kThreads) k_isl_mark_big(const uint32_t* __res
                                                            const uint32_t* __restrict__ islStart, const uint32_t* __restrict__ order,
                                                            const uint32_t* __restrict__ slotOf, uint8_t* __restrict__ big,
                                                            uint32_t* __restrict__ winFlag, uint32_t* __restrict__ blkFlag) {
-  const uint32_t nLeft = counts[1 + kIslandSlots];
+  const uint32_t nLeft = counts[1 + kIslandLists];
   for (uint32_t k = blockIdx.x; k < nLeft; k += gridDim.x) {
     const uint32_t isl = list[k];
     const uint32_t s0 = islStart[isl], m = islStart[isl + 1] - s0;
@@ -1037,32 +1071,24 @@ __global__ void __launch_bounds__(kBigTeam) k_island_pcg_big(IslandArgs a, uint3
 
 // ------------------------------------------------------------------------------------------------- host -----
 namespace {
-struct TierConfig { int team, rpt; IslandCaps caps; };
-// caps: nodes, matrix entries, inverse floats, blocks resident in shared memory
-const TierConfig kTiers[kIslandSlots] = {
-    {32, 1, {32u, 640u, 576u, 4u}},         // k_island_direct
-    {320, 2, {640u, 6656u, 9216u, 96u}},
-    {512, 2, {1024u, 12288u, 17408u, 192u}},
-    {1024, 0, {7168u, 0u, 0u, 0u}},         // k_island_pcg_big
-    {128, 2, {256u, 2816u, 3456u, 32u}},    // kSmallCtaSlot: 43 KB of shared memory
-    {128, 1, {kDenseMax, 0u, 0u, 0u}},      // kDenseSlot: k_island_invert<128> + k_island_dense<128>
-    {192, 1, {kDenseMax2, 0u, 0u, 0u}},     // kDenseSlot2: the same with N = 192
-};
-// Test hook: PIES_B200_ISLAND_MAXBLOCKS=k shrinks the shared-memory block tables of the CTA tiers to k entries, so islands
+// grid of list l for `units` CTAs of work
+int listGrid(int l, uint32_t units) { return (int)std::min<uint32_t>(units, (uint32_t)kLists[l].ctasPerSm * kNumSMs); }
+// Test hook: PIES_B200_ISLAND_MAXBLOCKS=k shrinks the shared-memory block tables of the CG lists to k entries, so islands
 // with more preconditioner blocks exercise the from-global-memory path of the block-Jacobi apply.
-IslandCaps tierCaps(int t) {
-  IslandCaps c = kTiers[t].caps;
+IslandCaps pcgCaps(int l) {
+  IslandCaps c = kLists[l].caps;
   static const int forced = [] { const char* e = std::getenv("PIES_B200_ISLAND_MAXBLOCKS"); return e ? std::atoi(e) : -1; }();
-  if (forced > 0 && t >= 1 && c.maxBlocks) c.maxBlocks = std::min<uint32_t>(c.maxBlocks, (uint32_t)forced);
+  if (forced > 0 && c.maxBlocks) c.maxBlocks = std::min<uint32_t>(c.maxBlocks, (uint32_t)forced);
   return c;
 }
-// k_island_pcg: t: whose team size, shared-memory layout and capacities; list: which island list (the same unless a list
-// is handed to a larger team)
-template <typename K>
-void launchTier(K kernel, int t, int grid, cudaStream_t s, const IslandArgs& a, int list = -1) {
-  const IslandLayout L = islandLayout(kTiers[t].caps);
-  cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
-  kernel<<<grid, kTiers[t].team, L.total, s>>>(a, L, tierCaps(t), list < 0 ? t : list);
+// the arrays of the matrix, the contacts and the island order, as every island kernel reads them
+IslandArgs islandArgs(const IslandWork& w, const CsrMatrix& S, const ContactLists& c) {
+  IslandArgs a{};
+  a.counts = w.counts.p; a.tierList = w.tierList.p; a.tierDesc = w.tierDesc.p; a.listStride = w.nBodies;
+  a.islStart = w.islStart.p; a.order = w.order.p; a.pos = w.pos.p; a.nnzOff = w.nnzOff.p;
+  a.rowPtr = S.rowPtr; a.col = S.col; a.val = S.val; a.colRank = w.colRank.p; a.rankInBody = w.rankInBody.p;
+  a.cPtr = c.nUnique ? c.cPtr : nullptr; a.cCol = c.cCol; a.cVal = c.cVal; a.cDiag = (c.nTri || c.nodeWeights()) ? c.cDiag : nullptr;
+  return a;
 }
 }  // namespace
 
@@ -1091,21 +1117,20 @@ int uploadIslandStatics(IslandWork& w, cudaStream_t s, const HostSystem& y) {
 }
 
 int buildIslands(IslandWork& w, cudaStream_t s, uint32_t n, const CsrMatrix& S, const ContactLists& c,
-                 const uint32_t* slotOf, const uint32_t* blockCount, uint32_t nBlocksBound, uint32_t tiersEnabled,
-                 int* launches) {
+                 const uint32_t* slotOf, const uint32_t* blockCount, uint32_t nBlocksBound, uint32_t tuning, int* launches) {
   int L = 0;
   const uint32_t nB = w.nBodies;
-  for (int t = 0; t < kIslandSlots; ++t) w.tierCount[t] = 0;
+  for (uint32_t& k : w.listCount) k = 0;
   w.nLeftIslands = 0; w.nLeftNodes = 0; w.united = false;
   if (!n || !nB) return 0;
   ICHECK(w.parent.reserve(nB + 1)); ICHECK(w.keys.reserve(nB + 1)); ICHECK(w.tmpKeys.reserve(nB + 1));
   ICHECK(w.vals.reserve(nB + 1)); ICHECK(w.tmpVals.reserve(nB + 1)); ICHECK(w.heads.reserve(nB + 2));
   ICHECK(w.nodeOff.reserve(nB + 2)); ICHECK(w.posOfBody.reserve(nB + 1)); ICHECK(w.islStart.reserve(nB + 2));
   ICHECK(w.order.reserve(n + 1)); ICHECK(w.pos.reserve(n + 1)); ICHECK(w.nnzOff.reserve(n + 2));
-  ICHECK(w.tierList.reserve((size_t)(kIslandSlots + 1) * nB)); ICHECK(w.tierDesc.reserve((size_t)(kIslandSlots + 1) * nB)); ICHECK(w.counts.reserve(16));
+  ICHECK(w.tierList.reserve((size_t)(kIslandLists + 1) * nB)); ICHECK(w.tierDesc.reserve((size_t)(kIslandLists + 1) * nB)); ICHECK(w.counts.reserve(16));
   ICHECK(w.blkLocal.reserve((size_t)nBlocksBound * 32 + 32)); ICHECK(w.slotIsl.reserve(n + 1));
   static const bool traceOn = std::getenv("PIES_B200_ISLAND_TRACE") != nullptr;
-  if (traceOn) ICHECK(w.trace.reserve((size_t)(kIslandSlots + 1) * nB));
+  if (traceOn) ICHECK(w.trace.reserve((size_t)(kIslandLists + 1) * nB));
   ICHECK(w.sortHist.reserve(sortHistBytes(nB) / 4 + 4));
   w.scanCap = std::max<uint64_t>(w.scanCap, std::max<uint64_t>(n, nB) + 2);
   ICHECK(w.scanScratch.reserve(scanScratchElems(w.scanCap)));
@@ -1126,29 +1151,31 @@ int buildIslands(IslandWork& w, cudaStream_t s, uint32_t n, const CsrMatrix& S, 
   k_isl_nodes<<<gridFor(n + 1, kThreads), kThreads, 0, s>>>(n, w.bodyOf.p, w.rankInBody.p, w.posOfBody.p, w.nodeOff.p, S.rowPtr,
                                                            c.nUnique ? c.cPtr : nullptr, w.order.p, w.pos.p, w.nnzOff.p); ++L;
   L += launchExclusiveScan(s, w.nnzOff.p, n + 1, w.scanScratch.p);
-  IslandTierTable tt;
-  for (int t = 0; t < kIslandSlots; ++t) tt.caps[t] = kTiers[t].caps;
-  static const bool noSmallCta = std::getenv("PIES_B200_NO_SMALL_CTA") != nullptr;   // A/B switch: tier 1 as one 320-thread list
-  static const bool noDense = std::getenv("PIES_B200_NO_DENSE") != nullptr;            // A/B switch: no dense-inverse list
-  if (noSmallCta) tt.caps[kSmallCtaSlot].maxNodes = 0;
-  static const bool noDense2 = std::getenv("PIES_B200_NO_DENSE2") != nullptr;          // A/B switch: dense list only up to 128 nodes
-  if (noDense) { tt.caps[kDenseSlot].maxNodes = 0; tt.caps[kDenseSlot2].maxNodes = 0; }
-  if (noDense2) tt.caps[kDenseSlot2].maxNodes = 0;
-  tt.enabled = tiersEnabled;
+  static const uint32_t switchedOff = (std::getenv("PIES_B200_NO_SMALL_CTA") ? kNoSmallCta : 0u) |
+                                      (std::getenv("PIES_B200_NO_DENSE") ? kNoDense : 0u) |
+                                      (std::getenv("PIES_B200_NO_DENSE2") ? kNoDense2 : 0u);
+  IslandClassifyTable tt;
+  for (int o = 0; o < kIslandLists; ++o) {
+    tt.id[o] = kClassifyOrder[o];
+    tt.list[o] = kLists[tt.id[o]];
+    if (tt.list[o].offBy & switchedOff) tt.list[o].caps.maxNodes = 0;
+  }
+  // Tuning bits: 4 = no island-local solve, 16 << t = public tier t off, 256 = tier 3 on.  Tier 3 is opt-in: a handful of
+  // its islands keep single SMs busy for milliseconds, the grid-wide CG spreads them over the whole device.
+  const uint32_t avail = (tuning & 256u) ? 0xFu : 0x7u;
+  tt.tiersOn = (tuning & 4u) ? 0u : (avail & ~((tuning >> 4) & 0xFu));
   k_isl_classify<<<gridFor(nB, kThreads), kThreads, 0, s>>>(w.counts.p, tt, w.islStart.p, w.nnzOff.p, w.order.p, slotOf, blockCount,
                                                            nB, w.tierList.p, w.tierDesc.p, w.counts.p); ++L;
   ICHECK(cudaMemcpyAsync(w.host, w.counts.p, 12 * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
   ICHECK(cudaEventRecord(w.ready, s));
   ICHECK(cudaEventSynchronize(w.ready));
-  for (int t = 0; t < kIslandSlots; ++t) w.tierCount[t] = w.host[1 + t];
-  w.nLeftIslands = w.host[1 + kIslandSlots];
-  w.nLeftNodes = w.host[2 + kIslandSlots];
-  w.inverseFloats = w.host[3 + kIslandSlots];
+  for (int l = 0; l < kIslandLists; ++l) w.listCount[l] = w.host[1 + l];
+  w.nLeftIslands = w.host[1 + kIslandLists];
+  w.nLeftNodes = w.host[2 + kIslandLists];
+  w.inverseFloats = w.host[3 + kIslandLists];
   // Both kinds present: the grid-wide CG only has to run over the rows of the left-over islands.
   w.restricted = false;
-  bool anyLocal = false;
-  for (int t = 0; t < kIslandSlots; ++t) anyLocal = anyLocal || w.tierCount[t];
-  if (w.nLeftIslands && anyLocal) {
+  if (w.nLeftIslands && w.anyLocal()) {
     const uint32_t nWin = (n + 255u) / 256u;
     ICHECK(w.big.reserve(n + 1)); ICHECK(w.winFlag.reserve(nWin + 2)); ICHECK(w.blkFlag.reserve(nBlocksBound + 2));
     ICHECK(w.actWin.reserve(nWin + 1)); ICHECK(w.actBlk.reserve(nBlocksBound + 1)); ICHECK(w.actCounts.reserve(4));
@@ -1158,50 +1185,47 @@ int buildIslands(IslandWork& w, cudaStream_t s, uint32_t n, const CsrMatrix& S, 
     ICHECK(cudaMemsetAsync(w.winFlag.p, 0, (nWin + 2) * sizeof(uint32_t), s));
     ICHECK(cudaMemsetAsync(w.blkFlag.p, 0, ((size_t)nBlocksBound + 2) * sizeof(uint32_t), s));
     k_isl_mark_big<<<(int)std::min<uint32_t>(w.nLeftIslands, 4 * kNumSMs), kThreads, 0, s>>>(
-        w.counts.p, w.tierList.p + (size_t)kIslandSlots * nB, w.islStart.p, w.order.p, slotOf, w.big.p, w.winFlag.p, w.blkFlag.p); ++L;
+        w.counts.p, w.tierList.p + (size_t)kIslandLists * nB, w.islStart.p, w.order.p, slotOf, w.big.p, w.winFlag.p, w.blkFlag.p); ++L;
     L += launchExclusiveScan(s, w.winFlag.p, nWin + 1, w.scanScratch.p);
     k_isl_compact<<<gridFor(nWin + 1, kThreads), kThreads, 0, s>>>(nWin, w.winFlag.p, w.actWin.p, w.actCounts.p); ++L;
     L += launchExclusiveScan(s, w.blkFlag.p, (uint64_t)nBlocksBound + 1, w.scanScratch.p);
     k_isl_compact<<<gridFor((uint64_t)nBlocksBound + 1, kThreads), kThreads, 0, s>>>(nBlocksBound, w.blkFlag.p, w.actBlk.p, w.actCounts.p + 1); ++L;
     w.restricted = true;
   }
-  if (w.tierCount[3]) {  // tier 3 keeps an island-local copy of the matrix in global memory
-    const size_t nnz = S.nnz + 6ull * c.nUnique + 16;
-    ICHECK(w.matCol.reserve(nnz)); ICHECK(w.matVal.reserve(nnz));
-  }
-  if (w.tierCount[kDenseSlot] || w.tierCount[kDenseSlot2]) {  // the dense lists: this substep's inverses
-    IslandArgs a{};
-    a.counts = w.counts.p; a.tierDesc = w.tierDesc.p; a.listStride = w.nBodies;
-    a.order = w.order.p; a.pos = w.pos.p; a.rowPtr = S.rowPtr; a.val = S.val; a.colRank = w.colRank.p; a.rankInBody = w.rankInBody.p;
-    a.cPtr = c.nUnique ? c.cPtr : nullptr; a.cCol = c.cCol; a.cVal = c.cVal; a.cDiag = (c.nTri || c.nodeWeights()) ? c.cDiag : nullptr;
-    if (w.tierCount[kDenseSlot]) ICHECK(w.denseInv.reserve((size_t)w.tierCount[kDenseSlot] * kDenseMax * kDenseMax));
-    if (w.tierCount[kDenseSlot2]) ICHECK(w.denseInv2.reserve((size_t)w.tierCount[kDenseSlot2] * kDenseMax2 * kDenseMax2));
-    // On the solver's stream: run beside the first local step on a side stream (r02x) they only moved their time from one
-    // phase to the other — both want every SM — and blurred the per-kernel timings of that step.
-    if (w.tierCount[kDenseSlot2]) {   // the longer inversions first
-      const uint32_t nd = w.tierCount[kDenseSlot2];
-      const size_t smem = ((size_t)kDenseMax2 * (kDenseMax2 + 4) + 4 * kDenseMax2) * sizeof(float);
-      cudaFuncSetAttribute(k_island_invert<(int)kDenseMax2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      k_island_invert<(int)kDenseMax2><<<(int)std::min<uint32_t>(nd, kNumSMs), (kDenseMax2 / 8) * (kDenseMax2 / 8), smem, s>>>(a, w.denseInv2.p, kDenseSlot2); ++L;
-    }
-    if (w.tierCount[kDenseSlot]) {
-      const uint32_t nd = w.tierCount[kDenseSlot];
-      const size_t smem = ((size_t)kDenseMax * (kDenseMax + 4) + 4 * kDenseMax) * sizeof(float);
-      cudaFuncSetAttribute(k_island_invert<(int)kDenseMax>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      k_island_invert<(int)kDenseMax><<<(int)std::min<uint32_t>(nd, 2 * kNumSMs), (kDenseMax / 8) * (kDenseMax / 8), smem, s>>>(a, w.denseInv.p, kDenseSlot); ++L;
+  // What the lists need before the first solve of the substep, in launch order (the longer inversions first)
+  const IslandArgs a = islandArgs(w, S, c);
+  for (const int l : kLaunchOrder) {
+    const uint32_t count = w.listCount[l], N = kLists[l].caps.maxNodes;
+    if (!count) continue;
+    if (kLists[l].kind == kBig) {   // an island-local copy of the matrix in global memory
+      const size_t nnz = S.nnz + 6ull * c.nUnique + 16;
+      ICHECK(w.matCol.reserve(nnz)); ICHECK(w.matVal.reserve(nnz));
+    } else if (kLists[l].kind == kDense) {
+      // The inverses, on the solver's stream: run beside the first local step on a side stream (r02x) they only moved
+      // their time from one phase to the other — both want every SM — and blurred the per-kernel timings of that step.
+      // One CTA of (N/8)^2 threads per island, as many per SM as the kernel's launch bounds.
+      ICHECK(w.denseInv[l].reserve((size_t)count * N * N));
+      const auto kernel = N == kDenseMax ? k_island_invert<(int)kDenseMax> : k_island_invert<(int)kDenseMax2>;
+      const size_t smem = ((size_t)N * (N + 4) + 4 * N) * sizeof(float);
+      cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+      kernel<<<(int)std::min<uint32_t>(count, (N <= 128 ? 2 : 1) * kNumSMs), (N / 8) * (N / 8), smem, s>>>(a, w.denseInv[l].p, l); ++L;
     }
   }
   if (launches) *launches += L;
   return 0;
 }
 
+void islandStats(const IslandWork& w, PiesB200Stats& st) {
+  for (uint32_t& k : st.islandsTier) k = 0;
+  for (int l = 0; l < kIslandLists; ++l) st.islandsTier[kLists[l].tier] += w.listCount[l];
+  st.islandsGlobal = w.nLeftIslands;
+  st.islandNodesGlobal = w.nLeftNodes;
+  st.islandInverseFloats = w.inverseFloats;
+}
+
 int launchIslandSolve(IslandWork& w, cudaStream_t s, const CsrMatrix& S, const ContactLists& c, const PcgWork& pw,
                       const uint32_t* slotOf, const float4* b, float4* x, float tol, uint32_t maxIter, uint32_t statSlot) {
-  IslandArgs a{};
-  a.counts = w.counts.p; a.tierList = w.tierList.p; a.tierDesc = w.tierDesc.p; a.listStride = w.nBodies;
-  a.islStart = w.islStart.p; a.order = w.order.p; a.pos = w.pos.p; a.nnzOff = w.nnzOff.p;
-  a.rowPtr = S.rowPtr; a.col = S.col; a.val = S.val; a.colRank = w.colRank.p; a.rankInBody = w.rankInBody.p;
-  a.cPtr = c.nUnique ? c.cPtr : nullptr; a.cCol = c.cCol; a.cVal = c.cVal; a.cDiag = (c.nTri || c.nodeWeights()) ? c.cDiag : nullptr;
+  IslandArgs a = islandArgs(w, S, c);
   a.slotOf = slotOf; a.blockNodes = pw.blockNodes; a.blockInv = pw.blockInv; a.blockMeta = pw.blockMeta;
   a.blkLocal = w.blkLocal.p; a.matCol = w.matCol.p; a.matVal = w.matVal.p; a.deltaScratch = pw.delta;
   a.apScratch = pw.ap; a.zScratch = pw.z; a.slotIsl = w.slotIsl.p;
@@ -1210,47 +1234,42 @@ int launchIslandSolve(IslandWork& w, cudaStream_t s, const CsrMatrix& S, const C
   int L = 0;
   // The lists of one solve are independent: the first one enqueued runs on the solver's stream, every further one on a
   // stream of its own beside it (the handful of long-running islands of tiers 2 and 3 next to the thousands of small ones
-  // that fill the other SMs; the warp tier in the SMs a CTA tier's last, partly filled wave leaves idle).  The longest
-  // chains are enqueued first.
+  // that fill the other SMs; the warp list in the SMs a CTA list's last, partly filled wave leaves idle).
   int present = 0;
-  for (int t = 0; t < kIslandSlots; ++t) present += w.tierCount[t] ? 1 : 0;
+  for (uint32_t k : w.listCount) present += k ? 1 : 0;
   if (present > 1) cudaEventRecord(w.fork, s);   // before anything of this solve is enqueued on s
   int used = 0;
-  bool first = true;
-  auto nextStream = [&]() -> cudaStream_t {
-    if (first) { first = false; return s; }
-    cudaStream_t st = w.aux[used++];
-    cudaStreamWaitEvent(st, w.fork, 0);
-    return st;
-  };
-  if (w.tierCount[3]) {
-    const uint32_t maxNodes = kTiers[3].caps.maxNodes;
-    const size_t smem = 32ull * maxNodes + 2 * 9 * 32 * sizeof(float);
-    cudaFuncSetAttribute(k_island_pcg_big, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k_island_pcg_big<<<(int)std::min<uint32_t>(w.tierCount[3], kNumSMs), kBigTeam, smem, nextStream()>>>(a, maxNodes, 3);
-    ++L;
-  }
-  if (w.tierCount[2]) { launchTier(k_island_pcg<512, 2>, 2, (int)std::min<uint32_t>(w.tierCount[2], kNumSMs), nextStream(), a); ++L; }
-  if (w.tierCount[1]) { launchTier(k_island_pcg<320, 2>, 1, (int)std::min<uint32_t>(w.tierCount[1], 2 * kNumSMs), nextStream(), a); ++L; }
-  if (w.tierCount[kSmallCtaSlot]) {
-    // A short list is latency bound (the solve waits for its slowest island, one warp per scheduler has nothing to hide
-    // a dependent shared-memory load behind): the 320-thread team gives every row its own thread.  A long list is
-    // throughput bound: five 128-thread CTAs per SM.
-    const uint32_t ns = w.tierCount[kSmallCtaSlot];
-    if (ns <= 2u * kNumSMs) launchTier(k_island_pcg<320, 2>, 1, (int)ns, nextStream(), a, kSmallCtaSlot);
-    else launchTier(k_island_pcg<128, 2>, kSmallCtaSlot, (int)std::min<uint32_t>(ns, 5 * kNumSMs), nextStream(), a);
-    ++L;
-  }
-  if (w.tierCount[kDenseSlot2]) {
-    k_island_dense<(int)kDenseMax2><<<(int)std::min<uint32_t>(w.tierCount[kDenseSlot2], 10 * kNumSMs), (int)kDenseMax2, 0, nextStream()>>>(a, w.denseInv2.p, kDenseSlot2);
-    ++L;
-  }
-  if (w.tierCount[kDenseSlot]) {
-    k_island_dense<(int)kDenseMax><<<(int)std::min<uint32_t>(w.tierCount[kDenseSlot], 16 * kNumSMs), (int)kDenseMax, 0, nextStream()>>>(a, w.denseInv.p, kDenseSlot);
-    ++L;
-  }
-  if (w.tierCount[0]) {
-    k_island_direct<<<(int)std::min<uint32_t>((w.tierCount[0] + 7) / 8, 4 * kNumSMs), 256, 0, nextStream()>>>(a, 0);
+  for (const int l : kLaunchOrder) {
+    const uint32_t count = w.listCount[l];
+    if (!count) continue;
+    cudaStream_t st = s;   // the first list enqueued
+    if (L) { st = w.aux[used++]; cudaStreamWaitEvent(st, w.fork, 0); }
+    const IslandList& e = kLists[l];
+    switch (e.kind) {
+      case kDirect:   // eight warps per CTA
+        k_island_direct<<<listGrid(l, (count + 7) / 8), 256, 0, st>>>(a, l);
+        break;
+      case kDense: {
+        const auto kernel = e.caps.maxNodes == kDenseMax ? k_island_dense<(int)kDenseMax> : k_island_dense<(int)kDenseMax2>;
+        kernel<<<listGrid(l, count), e.team, 0, st>>>(a, w.denseInv[l].p, l);
+        break;
+      }
+      case kCtaCg: {   // t: the list whose team, shared-memory layout and caps solve list l
+        const int t = count <= (uint32_t)kLists[e.shortList].ctasPerSm * kNumSMs ? e.shortList : l;
+        const IslandList& h = kLists[t];
+        const auto kernel = h.team == 128 ? k_island_pcg<128, 2> : (h.team == 320 ? k_island_pcg<320, 2> : k_island_pcg<512, 2>);
+        const IslandLayout lay = islandLayout(h.caps);
+        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total);
+        kernel<<<listGrid(t, count), h.team, lay.total, st>>>(a, lay, pcgCaps(t), l);
+        break;
+      }
+      case kBig: {
+        const size_t smem = 32ull * e.caps.maxNodes + 2 * 9 * 32 * sizeof(float);
+        cudaFuncSetAttribute(k_island_pcg_big, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        k_island_pcg_big<<<listGrid(l, count), kBigTeam, smem, st>>>(a, e.caps.maxNodes, l);
+        break;
+      }
+    }
     ++L;
   }
   for (int k = 0; k < used; ++k) { cudaEventRecord(w.join[k], w.aux[k]); cudaStreamWaitEvent(s, w.join[k], 0); }
