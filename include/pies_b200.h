@@ -221,6 +221,38 @@ int pies_b200_set_drag_targets(PiesB200Solver* s, uint32_t n, const uint32_t* no
 int pies_b200_raycast(PiesB200Solver* s, uint32_t nRays, const float* origins /* 3 per ray */, const float* dirs /* 3 per ray */,
                       const float* tMax, int32_t* tri, float* t, float* uv /* 2 per ray */);
 
+/* ---- [additive] external forces (DESIGN.md section 11): per-node forces a host applies, and a uniform wind acting on the
+ *      triangles.  Gravity stays as it is; the external force f_i of node i joins it where it acts:
+ *        PD:  the velocity update, v_i = [the reference's expression] + (h f_i) invMass_i, so f moves the next
+ *             substep's prediction, like gravity;
+ *        PBD: the advection, x_i = [the reference's expression] + ((f_i invMass_i) dt) dt.
+ *      (h = dt = fixedTimestepSize / timeSubsteps; each added operation rounded on its own.)  A node with invMass = 0
+ *      gains nothing.  f_i is evaluated once per substep, on the positions x and velocities v at the substep start:
+ *        f_i = hostForce_i + sum over the triangles t containing i, in ascending index order, of f_t / 3.
+ *      Wind velocity w, normal and tangential drag coefficients c_n, c_t >= 0; for triangle t = (a, b, c), every
+ *      operation rounded on its own (order in DESIGN.md section 11):
+ *        m = cross(x_b - x_a, x_c - x_a); |m| = 0 -> f_t = 0;  A = |m| / 2,  n = m / |m|
+ *        u = (v_a + v_b + v_c) / 3 - w;  un = dot(u, n),  ut = u - un n
+ *        f_t = -A (c_n un |un| n + c_t ut)     (the same for either winding)
+ *      Only triangles feel the wind: ropes, bare nodes and bodies without triangles do not.  The integration is explicit
+ *      and not clamped: keep h c_n A_i |un| invMass_i well below 1 (A_i = the area of node i's triangles / 3), and
+ *      likewise h c_t A_i invMass_i, or the drag overshoots and the body gains energy.
+ *      Neither forces nor wind are counted in PiesB200Stats.  Without either, every kernel computes what it computed
+ *      before external forces existed. */
+/* Replaces the host forces (3 floats per node, n = 0 removes them).  The set persists across ticks until replaced, stays
+ * valid when bodies are appended (new nodes get none), and pies_b200_clear removes it.  The arrays are copied before the
+ * call returns.  EINVAL: a node id >= vertex_count(), a duplicate id, a non-finite component, a null array with n > 0, or
+ * a call inside pd_tick_begin .. pd_tick_end; a rejected set leaves the previous one in place. */
+int pies_b200_set_external_forces(PiesB200Solver* s, uint32_t n, const uint32_t* nodes, const float* forces /* 3n */);
+/* Sets the wind: velocity (3 floats), c_n = normalDrag, c_t = tangentialDrag.  Both coefficients 0 remove it, and so does
+ * pies_b200_clear.  EINVAL: a null velocity, a non-finite value, a negative coefficient, or a call inside
+ * pd_tick_begin .. pd_tick_end; a rejected call leaves the previous wind in place. */
+int pies_b200_set_wind(PiesB200Solver* s, const float* velocity /* 3 */, float normalDrag, float tangentialDrag);
+/* f_i of every node (3 floats per node, vertex_count() nodes) as applied in the last substep of the last tick, gravity
+ * not included.  All zeros when that tick had neither forces nor wind, before the first tick and after clear; nodes
+ * appended since that tick read 0. */
+int pies_b200_get_external_forces(PiesB200Solver* s, float* xyz);
+
 /* ---- readback (Solver::getVertices/getLines/getTriangles; Solver.h:65-69) ---- */
 uint32_t pies_b200_vertex_count(const PiesB200Solver* s);
 uint32_t pies_b200_line_index_count(const PiesB200Solver* s);

@@ -183,6 +183,7 @@ int pies_b200_clear(PiesB200Solver* s) {
     s->stats.collisionProjections = 0;
     s->colliderSet.clear(); s->colMaskColliders = 0;
     s->dragCount = 0;
+    pies::clearForces(s);
     s->renderStateDirty = true;
     return PIES_B200_OK;
   });
@@ -438,6 +439,15 @@ int pies_b200_get_collider_contacts(PiesB200Solver* s, uint32_t* masks) {
 }
 int pies_b200_set_drag_targets(PiesB200Solver* s, uint32_t n, const uint32_t* nodes, const float* targets, const float* weights) {
   return guarded(s, [&]() { return pies::setDragTargets(s, n, nodes, targets, weights); });
+}
+int pies_b200_set_external_forces(PiesB200Solver* s, uint32_t n, const uint32_t* nodes, const float* forces) {
+  return guarded(s, [&]() { return pies::setExternalForces(s, n, nodes, forces); });
+}
+int pies_b200_set_wind(PiesB200Solver* s, const float* velocity, float normalDrag, float tangentialDrag) {
+  return guarded(s, [&]() { return pies::setWind(s, velocity, normalDrag, tangentialDrag); });
+}
+int pies_b200_get_external_forces(PiesB200Solver* s, float* xyz) {
+  return guarded(s, [&]() { return pies::getExternalForces(s, xyz); });
 }
 int pies_b200_raycast(PiesB200Solver* s, uint32_t nRays, const float* origins, const float* dirs, const float* tMax,
                       int32_t* tri, float* t, float* uv) {

@@ -432,6 +432,7 @@ int pdTickBegin(PiesB200Solver* s) {
   c->launches0 = s->launches;
   s->pdCtx = c;
   if (!s->n) return PIES_B200_OK;
+  if ((rc = prepareForces(s))) { pdAbort(s); return rc; }
   if (s->islands) {
     const size_t words = 4ull * s->opt.timeSubsteps * s->opt.iterations + 4;
     PIES_CHECK(s, s->islands->solveStats.reserve(words));
@@ -461,6 +462,7 @@ int pdSubstepBegin(PiesB200Solver* s) {
   PhaseTimer& timer = c->timer;
   int rc;
   timer.begin(kPhOther);
+  s->launches += launchForces(st, n, forceSet(s), s->q.p, s->vel.p);   // on the substep-start q and vel
   s->launches += launchPredict(st, n, s->q.p, s->vel.p, s->msn.p, h);
   timer.end();
 
@@ -652,7 +654,7 @@ int pdSubstepEnd(PiesB200Solver* s) {
     s->stats.reserved = std::min(s->blocks->host[1], 65535u) | (std::min(s->blocks->host[2], 65535u) << 16);
   }
   timer.begin(kPhOther);
-  s->launches += launchVelocityUpdate(st, n, s->q.p, s->prev.p, s->vel.p, h, o.damping, o.gravity);
+  s->launches += launchVelocityUpdate(st, n, s->q.p, s->prev.p, s->vel.p, h, o.damping, o.gravity, forceSet(s).field());
   timer.end();
   timer.begin(kPhContact);
   if (s->contact) s->launches += launchFriction(st, *s->contact, lists, n, s->q.p, s->vel.p, o.friction, o.staticFrictionThreshold);

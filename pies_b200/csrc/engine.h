@@ -117,6 +117,18 @@ struct PiesB200Solver {
   // drag targets (pick.cu): the validated set's size and its device copy (node ids, (g, w)); dragCount = 0 = none
   uint32_t dragCount = 0;
   pies::DevBuf<uint32_t> dragNode; pies::DevBuf<float4> dragTargetW;
+  // external forces (forces.cu): the validated host set (copied by set_external_forces; uploaded as the dense per-node
+  // buffer hostForce, zeros for unlisted nodes, at the first tick after a change or a node-count change), the wind
+  // (wind = (velocity, c_n), windTangential = c_t; both coefficients 0 = none) with its node -> triangle CSR of topology
+  // windCsrVersion, per-triangle slots and per-node sums (allocated at the first tick with wind), and what the last tick
+  // applied: forceMode bit 1 = hostForce, bit 2 = wind (fext), for forceModeN nodes
+  std::vector<uint32_t> forceIds; std::vector<float4> forceVals;
+  bool forceDirty = false; uint32_t forceDenseN = 0;
+  pies::DevBuf<float4> hostForce;
+  float4 wind{0.0f, 0.0f, 0.0f, 0.0f}; float windTangential = 0.0f;
+  uint64_t windCsrVersion = ~0ull;
+  pies::DevBuf<int> windPtr; pies::DevBuf<uint32_t> windList; pies::DevBuf<float4> windSlot, fext;
+  uint32_t forceMode = 0, forceModeN = 0;
   // raycast staging (pick.cu): rays (2 float4 each), per-ray hit keys, packed results
   pies::DevBuf<float4> rays; pies::DevBuf<unsigned long long> rayKey; pies::DevBuf<float4> rayHit;
 
@@ -161,6 +173,21 @@ int setColliders(PiesB200Solver* s, uint32_t n, const PiesB200Collider* c);
 inline ColliderSet colliderSet(const PiesB200Solver* s) { return ColliderSet{s->colliders.p, (uint32_t)s->colliderSet.size()}; }
 int setDragTargets(PiesB200Solver* s, uint32_t n, const uint32_t* nodes, const float* targets, const float* weights);
 inline DragSet dragSet(const PiesB200Solver* s) { return DragSet{s->dragNode.p, s->dragTargetW.p, s->dragCount}; }
+int setExternalForces(PiesB200Solver* s, uint32_t n, const uint32_t* nodes, const float* forces);
+int setWind(PiesB200Solver* s, const float* velocity, float normalDrag, float tangentialDrag);
+int prepareForces(PiesB200Solver* s);   // tick start, after ensureBuilt
+int getExternalForces(PiesB200Solver* s, float* xyz);
+void clearForces(PiesB200Solver* s);
+// the forces the current (or last) tick applies, as fixed by prepareForces
+inline ForceSet forceSet(const PiesB200Solver* s) {
+  ForceSet f;
+  if (s->forceMode & 1u) f.host = s->hostForce.p;
+  if (s->forceMode & 2u) {
+    f.nTri = s->scene.triCount(); f.tri = s->triIds.p; f.ptr = s->windPtr.p; f.list = s->windList.p;
+    f.slot = s->windSlot.p; f.fext = s->fext.p; f.wind = s->wind; f.ct = s->windTangential;
+  }
+  return f;
+}
 int raycast(PiesB200Solver* s, uint32_t nRays, const float* origins, const float* dirs, const float* tMax, int32_t* tri,
             float* t, float* uv);
 int pbdOccupancyCounts(PiesB200Solver* s, uint64_t* nCells, uint64_t* nMembers);

@@ -107,8 +107,9 @@ int launchGatherRhs(cudaStream_t s, uint32_t n, const uint32_t* nodes, const flo
 // Fused tet projections + RHS of every node of the segments (with the collision and floor terms of c when it has any).
 int launchTetRhs(cudaStream_t s, const TetElems& e, const TetSegments& sg, const float4* q, const float4* msn,
                  const int* incPtr, const ContactLists& c, const float4* contribC, float4* snap, float4* rhs);
+// fext: per-node external force (ForceSet::field()), null = none: the parent's k_velocity
 int launchVelocityUpdate(cudaStream_t s, uint32_t n, const float4* q, float4* prev, float4* vel, float h,
-                         float damping, float gravity);
+                         float damping, float gravity, const float4* fext);
 
 // ------------------------------------------------------ static colliders -----
 // (colliders.cu; col = the solver's device copy of its colliders, n of them)
@@ -137,6 +138,21 @@ struct DragSet { const uint32_t* node = nullptr; const float4* targetW = nullptr
 int launchDragTerms(cudaStream_t s, const DragSet& d, float* floorW, float4* msn);
 // PBD, after the position-constraint sweep: x += min(w, 1) (g - x).
 int launchPbdDrag(cudaStream_t s, const DragSet& d, float4* q);
+
+// ------------------------------------------------------- external forces -----
+// (forces.cu) host: dense per-node host forces, or null.  nTri > 0: wind on the triangles tri (3 ids each) with
+// wind = (w, c_n) and c_t = ct, over the node -> triangle CSR (ptr, list), one slot per triangle, summed into fext.
+struct ForceSet {
+  const float4* host = nullptr;
+  uint32_t nTri = 0;
+  const uint32_t* tri = nullptr; const int* ptr = nullptr; const uint32_t* list = nullptr;
+  float4* slot = nullptr; float4* fext = nullptr;
+  float4 wind{0.0f, 0.0f, 0.0f, 0.0f}; float ct = 0.0f;
+  // what the velocity update (PD) or the advection (PBD) reads: null = no external force
+  const float4* field() const { return nTri ? fext : host; }
+};
+// Substep start, before k_predict / k_pbd_advect: k_wind_tri + k_force_gather into fext when nTri > 0, else nothing.
+int launchForces(cudaStream_t s, uint32_t n, const ForceSet& f, const float4* q, const float4* vel);
 
 // ------------------------------------------------------------------ PCG -----
 struct PcgWork {

@@ -77,8 +77,12 @@ void destroyPbdWork(PbdWork* w) {
 // ------------------------------------------------------------------------------------------
 // streaming kernels
 // advect (Solver.cpp:47-52): prev = pos; pos += v dt + (0,-g,0) dt dt
+// kForce adds the external force (forces.cu) as a final addition, ((f invMass) dt) dt; the variant without it is the
+// reference's advection and runs whenever the solver has no external force.
+template <bool kForce>
 __global__ void __launch_bounds__(kThreads) k_pbd_advect(uint32_t n, float4* __restrict__ q, float4* __restrict__ prev,
-                                                         const float4* __restrict__ vel, float dt, float gravity) {
+                                                         const float4* __restrict__ vel, float dt, float gravity,
+                                                         const float4* __restrict__ fext) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   float4 p = q[i], o = prev[i], v = vel[i];
@@ -87,6 +91,12 @@ __global__ void __launch_bounds__(kThreads) k_pbd_advect(uint32_t n, float4* __r
   p.x = ex::add(p.x, ex::add(ex::mul(v.x, dt), 0.0f));
   p.y = ex::add(p.y, ex::add(ex::mul(v.y, dt), gy));
   p.z = ex::add(p.z, ex::add(ex::mul(v.z, dt), 0.0f));
+  if constexpr (kForce) {
+    const float4 f = fext[i];
+    p.x = ex::add(p.x, ex::mul(ex::mul(ex::mul(f.x, p.w), dt), dt));
+    p.y = ex::add(p.y, ex::mul(ex::mul(ex::mul(f.y, p.w), dt), dt));
+    p.z = ex::add(p.z, ex::mul(ex::mul(ex::mul(f.z, p.w), dt), dt));
+  }
   q[i] = p;
 }
 
@@ -853,6 +863,7 @@ int tickPBD(PiesB200Solver* s, bool refreshMirror) {
   if (!s->pbd) s->pbd = new PbdWork();
   PbdWork& w = *s->pbd;
   if (w.builtVersion != s->scene.topologyVersion && (rc = buildPbd(s, w))) return rc;
+  if ((rc = prepareForces(s))) return rc;
   cudaStream_t st = s->stream;
   const PiesB200Options& o = s->opt;
   const float dt = o.fixedTimestepSize / (float)o.timeSubsteps;
@@ -864,8 +875,14 @@ int tickPBD(PiesB200Solver* s, bool refreshMirror) {
   PosOp pos{w.posIds.p, w.posTk.p, w.posTargetW.p};
   DistOp dist{w.distIds.p, w.distTk.p, w.distRestW.p};
   BendOp bend{w.bendIds.p, w.bendTk.p, w.bendAngleW.p};
+  const ForceSet forces = forceSet(s);
   for (uint32_t sub = 0; sub < o.timeSubsteps; ++sub) {
-    k_pbd_advect<<<gridFor(n, kThreads), kThreads, 0, st>>>(n, s->q.p, s->prev.p, s->vel.p, dt, o.gravity); ++s->launches;
+    s->launches += launchForces(st, n, forces, s->q.p, s->vel.p);
+    if (const float4* f = forces.field())
+      k_pbd_advect<true><<<gridFor(n, kThreads), kThreads, 0, st>>>(n, s->q.p, s->prev.p, s->vel.p, dt, o.gravity, f);
+    else
+      k_pbd_advect<false><<<gridFor(n, kThreads), kThreads, 0, st>>>(n, s->q.p, s->prev.p, s->vel.p, dt, o.gravity, nullptr);
+    ++s->launches;
     for (uint32_t it = 0; it < o.iterations; ++it) {
       if (!s->releaseHinge && (rc = sweep(s, w, w.nPos, pos))) goto done;
       s->launches += launchPbdDrag(st, dragSet(s), s->q.p);

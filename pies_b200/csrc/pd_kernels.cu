@@ -393,9 +393,13 @@ int launchGatherRhs(cudaStream_t s, uint32_t n, const uint32_t* nodes, const flo
 }
 
 // ---- velocity update (Solver.cpp:386-395) -----------------------------------------------------
+// kForce adds the external force (forces.cu) as a final addition, (h f) invMass, rounded on its own; the variant without
+// it is the reference's update and runs whenever the solver has no external force.
+template <bool kForce>
 __global__ void __launch_bounds__(kThreads) k_velocity(uint32_t n, const float4* __restrict__ q,
                                                        float4* __restrict__ prev, float4* __restrict__ vel,
-                                                       float h, float damping, float gravity) {
+                                                       float h, float damping, float gravity,
+                                                       const float4* __restrict__ fext) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   float4 p = q[i];
@@ -406,15 +410,22 @@ __global__ void __launch_bounds__(kThreads) k_velocity(uint32_t n, const float4*
   v.x = k * (p.x - pp.x) / h + h * 0.0f * p.w;
   v.y = k * (p.y - pp.y) / h + h * fy * p.w;
   v.z = k * (p.z - pp.z) / h + h * 0.0f * p.w;
+  if constexpr (kForce) {
+    const float4 f = ldStream(fext + i);
+    v.x = __fadd_rn(v.x, __fmul_rn(__fmul_rn(h, f.x), p.w));
+    v.y = __fadd_rn(v.y, __fmul_rn(__fmul_rn(h, f.y), p.w));
+    v.z = __fadd_rn(v.z, __fmul_rn(__fmul_rn(h, f.z), p.w));
+  }
   v.w = 0.0f;
   vel[i] = v;
   prev[i] = make_float4(p.x, p.y, p.z, pp.w);
 }
 
 int launchVelocityUpdate(cudaStream_t s, uint32_t n, const float4* q, float4* prev, float4* vel, float h,
-                         float damping, float gravity) {
+                         float damping, float gravity, const float4* fext) {
   if (!n) return 0;
-  k_velocity<<<gridFor(n, kThreads), kThreads, 0, s>>>(n, q, prev, vel, h, damping, gravity);
+  if (fext) k_velocity<true><<<gridFor(n, kThreads), kThreads, 0, s>>>(n, q, prev, vel, h, damping, gravity, fext);
+  else k_velocity<false><<<gridFor(n, kThreads), kThreads, 0, s>>>(n, q, prev, vel, h, damping, gravity, nullptr);
   return 1;
 }
 

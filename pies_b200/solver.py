@@ -199,6 +199,9 @@ _SIGNATURES = {
     "pies_b200_probe_colliders": (C.c_int, [C.c_uint32, _vp, C.c_uint32, _vp, _vp, _vp]),
     "pies_b200_set_drag_targets": (C.c_int, [_vp, C.c_uint32, _vp, _vp, _vp]),
     "pies_b200_raycast": (C.c_int, [_vp, C.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "pies_b200_set_external_forces": (C.c_int, [_vp, C.c_uint32, _vp, _vp]),
+    "pies_b200_set_wind": (C.c_int, [_vp, _vp, C.c_float, C.c_float]),
+    "pies_b200_get_external_forces": (C.c_int, [_vp, _vp]),
     "pies_b200_probe_segments": (C.c_int, [C.c_uint32, _vp, C.c_uint32, _vp, C.c_uint32, _vp, _u64p] + [_vp] * 7),
 }
 
@@ -519,6 +522,30 @@ class Solver:
         p = lambda a: a.ctypes.data_as(_vp) if a.size else None
         self._ck(lib().pies_b200_raycast(self.h, n, p(o), p(d), p(tm), p(tri), p(t), p(uv)))
         return tri, t, uv
+
+    def setExternalForces(self, nodes, forces):
+        """Replaces the host forces: node ids and their forces (n x 3), applied every substep until replaced.  Empty
+        arrays remove the set."""
+        ids = np.ascontiguousarray(nodes, dtype=np.uint32).reshape(-1)
+        f = np.ascontiguousarray(forces, dtype=np.float32).reshape(-1, 3)
+        if len(f) != len(ids):
+            raise ValueError("setExternalForces: %d nodes but %d forces" % (len(ids), len(f)))
+        p = lambda a: a.ctypes.data_as(_vp) if a.size else None
+        self._ck(lib().pies_b200_set_external_forces(self.h, len(ids), p(ids), p(f)))
+
+    def setWind(self, velocity, normalDrag, tangentialDrag):
+        """Sets a uniform wind acting on the triangles: its velocity (3,) and the normal and tangential drag coefficients
+        (both 0 removes it)."""
+        w = _v3(velocity)
+        self._ck(lib().pies_b200_set_wind(self.h, w.ctypes.data_as(_vp), normalDrag, tangentialDrag))
+
+    def externalForces(self):
+        """Per node, the external force (host force plus wind, gravity excluded) applied in the last substep of the
+        last tick: float32 (n, 3)."""
+        out = np.zeros((lib().pies_b200_vertex_count(self.h), 3), np.float32)
+        if len(out):
+            self._ck(lib().pies_b200_get_external_forces(self.h, out.ctypes.data_as(_vp)))
+        return out
 
     def staticCollisions(self):
         out = np.empty(lib().pies_b200_static_collision_count(self.h), dtype=np.uint32)
